@@ -1,14 +1,14 @@
 #!/usr/bin/env python
 """Benchmark of the appearance-flow training hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|3|4|5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|3|4|5] [--dump-outputs DIR]
 
 Own arm: one "step" = forward + backward + Adam of the single-view appearance-flow model on a
 synthetic 224x224 car-render batch of 64 per GPU (BASELINE configs[1]; data parallel over N
 GPUs = weak scaling, configs[2] shape of work per GPU), replayed from a captured CUDA graph.
-  value  : samples/s with the batch resident in HBM (CUDA events, max over ranks)
+  value  : samples/s with the batch resident in HBM (CUDA events, max over ranks), K timed steps
   e2e    : samples/s through the public API with pinned-host inputs copied H2D and the loss
-           read back D2H inside the timed region, every step
+           read back D2H inside the timed region, every step; K more timed steps
   roofline / sampler : the dominant kernel of the step and the standalone sampler kernels
            against MEASURED_PEAKS.json
   cpu_baseline : the oracle's torch-CPU port of the same step on the host cores (rank 0, N=1)
@@ -16,6 +16,8 @@ Reference arm (--impl reference): that CPU port alone, on a bounded batch-8 samp
 --config selects the BASELINE.json workload (default 2 = configs[1], the one the metric is quoted on; 3 = high-dim
 viewpoint variant, 4 = cars_colordepth RGB+depth with per-channel L1, 5 = 4 source frames + confidence fusion on the
 multi-object trunk); every one is 64 samples per GPU at 224x224, V=19, captured into one CUDA graph.
+--dump-outputs DIR writes what the last timed step computed on rank 0 to DIR/<name>.npy (dump_outputs()).  The inputs
+and initial weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -24,6 +26,7 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
@@ -290,6 +293,60 @@ def layer_gflop(B):
     return t
 
 
+# the outputs of a step that each benchmarked model class holds after train_step (as configured in WORKLOADS)
+DUMP_OUTPUTS = {"AppearanceFlowModel": ("flow_field", "gen"), "AppFlowHighDimAngle": ("flow_field", "gen"),
+                "Base_Prediction_Model": ("gen_image1", "gen_dimage1"),
+                "MultiViewFusionAppFlow": ("flow_field", "gens", "logits", "fused")}
+DUMP_MAX_OUTPUT = 1 << 21        # elements per output array (8 MB in float32)
+DUMP_MAX_PARAM = 1 << 18         # elements per parameter (1 MB); the FC matrices are 17M-51M elements
+DUMP_MAX_BYTES = 64 << 20
+
+
+def _dump_sample(t, cap, name):
+    """``t`` as a float32 array: whole when it has at most ``cap`` elements; otherwise ``cap`` of its flattened elements
+    at indices drawn without replacement from a generator seeded with ``name``, in ascending order -- the same indices
+    on every run and build."""
+    import numpy as np
+    import torch
+    x = t.detach()
+    if x.numel() > cap:
+        idx = np.sort(np.random.default_rng(zlib.crc32(name.encode())).choice(x.numel(), cap, replace=False))
+        x = x.reshape(-1)[torch.from_numpy(idx).to(x.device)]
+    return x.float().cpu().numpy()
+
+
+def dump_outputs(out_dir, model, loss, world, rank):
+    """What the last timed step computed, one ``out_dir/<name>.npy`` per array: ``loss`` (float64 scalar), the model's
+    outputs of that step (``gen``, ``flow_field``, ...; rank 0's shard of the batch under data parallelism) and every
+    parameter after the step's update (``param.<variable name with '/' -> '.'>``), float32.  Arrays larger than
+    DUMP_MAX_OUTPUT / DUMP_MAX_PARAM elements are written as the fixed seeded sample of _dump_sample().  Collective
+    under data parallelism: every rank calls it, rank 0 writes."""
+    import numpy as np
+    import torch
+    dp = getattr(model, "_dp", None)
+    if world > 1 and hasattr(dp, "gather_full_state"):
+        dp.gather_full_state()       # sharded: the fp32 masters live with their owning rank
+    else:
+        model.flush_updates()        # the late FC matrices' update of the last step may still be pending
+    torch.cuda.synchronize()
+    if rank != 0:
+        return
+    arrays = {"loss": np.asarray(loss, dtype=np.float64)}
+    for name in DUMP_OUTPUTS[type(model).__name__]:
+        t = getattr(model, name, None)
+        if not isinstance(t, torch.Tensor):
+            raise RuntimeError("%s holds no output %r after its train step" % (type(model).__name__, name))
+        arrays[name] = _dump_sample(t, DUMP_MAX_OUTPUT, name)
+    for name, v in model.store.vars.items():
+        key = "param." + name.replace("/", ".")
+        arrays[key] = _dump_sample(v.master, DUMP_MAX_PARAM, key)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, "dump of %d bytes exceeds %d" % (total, DUMP_MAX_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -302,7 +359,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-micro", action="store_true")
     ap.add_argument("--eager", action="store_true", help="do not capture a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss, outputs and updated parameters of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "own":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl own)")
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -329,7 +392,7 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
     pk = peaks()
     W = max(3, args.warmup)
-    K = max(1, args.steps)
+    K = args.steps
 
     cls_name, extra, workload, loss_name = WORKLOADS[args.config]
     conf = {"batch_size": BATCH, "learning_rate": 1e-4, "image_size": H, "viewpoint_dim": V, "loss": "l2", "seed": 0}
@@ -431,6 +494,8 @@ def main():
     barrier()
     ms_e2e = max(ee0.elapsed_time(ee1), 1e3 * (time.perf_counter() - t0)) / K
     clocks = sampler.summary() if sampler else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, model, last, world, rank)
     if world > 1:
         t = torch.tensor([ms, ms_e2e], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -1,0 +1,18 @@
+# Written for tests/test_host_logic.py in the format of the reference's tensorflowdata/*/conf.py (SURVEY.md section 5):
+# direct-regression multi-object model (multiobject_main_model.py), which this build does not implement.
+import os
+current_dir = os.path.dirname(os.path.realpath(__file__))
+from multiobject_main_model import Base_Prediction_Model
+
+configuration = {
+    'experiment_name': os.path.basename(current_dir),
+    'data_dir': current_dir + '/data',
+    'output_dir': current_dir + '/modeldata',
+    'current_dir': current_dir,
+    'num_iterations': 200000,
+    'batch_size': 64,
+    'learning_rate': 1e-4,
+    'train_val_split': 0.95,
+    'use_color': '',
+    'model': Base_Prediction_Model,
+}

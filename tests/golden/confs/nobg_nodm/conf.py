@@ -1,0 +1,15 @@
+# Written for tests/test_host_logic.py in the format of the reference's tensorflowdata/*/conf.py (SURVEY.md section 5):
+# an MV3D experiment: neither 'model' nor a colour / depth switch; it belongs to the mv3d scripts, not train.py.
+import os
+current_dir = os.path.dirname(os.path.realpath(__file__))
+
+configuration = {
+    'experiment_name': os.path.basename(current_dir),
+    'data_dir': current_dir + '/data',
+    'output_dir': current_dir + '/modeldata',
+    'current_dir': current_dir,
+    'num_iterations': 200000,
+    'batch_size': 64,
+    'learning_rate': 1e-4,
+    'train_val_split': 0.95,
+}

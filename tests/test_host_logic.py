@@ -140,7 +140,10 @@ def test_multiview_variable_table():
     assert m.INPUT_KEYS == ("image0", "depth0", "image0_mask0", "image0_mask1", "displacement", "image1")
 
 
-REF_CONFS = os.path.join(os.sep, "root", "reference", "tensorflowdata")
+# Experiment confs in the reference's tensorflowdata/<experiment>/conf.py format, one for every way train.py treats a
+# conf: each model class imported by the reference's module names, the Base_Prediction_Model fallback, the reference's
+# unparsable appflow_multiobject conf, the out-of-scope multiobject_main_model and an MV3D conf.
+REF_CONFS = os.path.join(ROOT, "tests", "golden", "confs")
 
 
 def _reference_confs():
@@ -151,11 +154,14 @@ def _reference_confs():
     return sorted(out)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CONFS), reason="the reference tree is only present in the authoring container")
+def test_reference_conf_fixtures_are_present():
+    assert len(_reference_confs()) == 9
+
+
 @pytest.mark.parametrize("rel", _reference_confs())
 def test_every_reference_conf_builds_its_model_and_step_plumbing(rel):
-    """train.py:40-65 on the UNMODIFIED reference conf files (meta device: variable tables and shapes only): the model
-    class the conf selects builds, and the driver's plumbing (input_spec / INPUT_KEYS / synthetic batches / checkpoint
+    """train.py:40-65 on conf files loaded unchanged (meta device: variable tables and shapes only): the model class
+    the conf selects builds, and the driver's plumbing (input_spec / INPUT_KEYS / synthetic batches / checkpoint
     surface) covers it.  Confs of out-of-scope model files fail with a clear import error."""
     from dynamic_multiview_3d_b200 import train
     from dynamic_multiview_3d_b200.model_base import ModelBase
