@@ -26,6 +26,7 @@ SIGNATURES = {
     "dmv_last_error": (_i, [C.c_char_p, _sz]),
     "dmv_launch_count": (_ll, []),
     "dmv_tc_launch_count": (_ll, []),
+    "dmv_launch_count_named": (_ll, [C.c_char_p]),
     "dmv_sampler_fwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _u, _vp]),
     "dmv_sampler_bwd_workspace_size": (_sz, [_i, _i, _i, _i, _i, _i]),
     "dmv_sampler_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _u, _vp, _sz, _vp]),
@@ -112,3 +113,8 @@ def launch_count():
 
 def tc_launch_count():
     return int(load().dmv_tc_launch_count())
+
+
+def launch_count_named(what):
+    """Launches so far of the kernel form labelled ``what`` (the label of its launch check in csrc/)."""
+    return int(load().dmv_launch_count_named(what.encode()))

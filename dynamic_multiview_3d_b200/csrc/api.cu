@@ -1,6 +1,8 @@
-// Library info, error state and the diagnostic launch counter of libdmv3d.
+// Library info, error state and the diagnostic launch counters of libdmv3d.
 #include <atomic>
+#include <mutex>
 #include <stdarg.h>
+#include <unordered_map>
 
 #include "common.cuh"
 
@@ -8,6 +10,15 @@ namespace dmv {
 static thread_local char g_err[512] = "";
 static std::atomic<long long> g_launches{0};
 static std::atomic<long long> g_tc_launches{0};
+// per-label counts, keyed by the label literal's address (the same text from two translation units may be two keys;
+// dmv_launch_count_named sums them by content)
+static std::mutex g_named_mu;
+static std::unordered_map<const char*, long long> g_named;
+
+void count_launch_named(const char* what) {
+    std::lock_guard<std::mutex> lk(g_named_mu);
+    ++g_named[what];
+}
 
 void set_error(const char* fmt, ...) {
     va_list ap;
@@ -31,4 +42,12 @@ int dmv_last_error(char* buf, size_t n) {
 }
 long long dmv_launch_count(void) { return dmv::g_launches.load(std::memory_order_relaxed); }
 long long dmv_tc_launch_count(void) { return dmv::tc_launches(); }
+long long dmv_launch_count_named(const char* what) {
+    if (!what) return 0;
+    std::lock_guard<std::mutex> lk(dmv::g_named_mu);
+    long long n = 0;
+    for (const auto& kv : dmv::g_named)
+        if (strcmp(kv.first, what) == 0) n += kv.second;
+    return n;
+}
 }

@@ -13,6 +13,7 @@ namespace dmv {
 
 void set_error(const char* fmt, ...);
 void count_launch(int n = 1);
+void count_launch_named(const char* what);      // what: a string literal (kept by address)
 void count_tc_launch();
 long long tc_launches();
 
@@ -21,7 +22,8 @@ inline int fail(int code, const char* msg) {
     return code;
 }
 
-// checks the launch that was just issued (async errors surface at the caller's next sync)
+// checks the launch that was just issued (async errors surface at the caller's next sync) and counts it under its
+// label (dmv_launch_count_named), so tests can tell which kernel form ran
 inline int check_launch(const char* what) {
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) {
@@ -29,6 +31,7 @@ inline int check_launch(const char* what) {
         return DMV_E_CUDA;
     }
     count_launch();
+    count_launch_named(what);
     return DMV_OK;
 }
 

@@ -67,7 +67,7 @@ size_t dmv_wgrad_workspace_size(int B, int H, int W, int Cbig, int Csmall, int k
     const long long pixels = (long long)B * ph.out * pw.out;
     const int taps = kh * kw;
     size_t a = simt_wgrad_workspace(taps, Cbig, Csmall, pixels);
-    size_t b = tc_wgrad_workspace(taps, Cbig, Csmall, pixels);
+    size_t b = tc_wgrad_workspace(taps, Cbig, Csmall, B, ph.out, pw.out);
     if (b > a) a = b;
     if (thin_side(Cbig)) {
         size_t c = tc_thin_workspace(B, H, W, Cbig, Csmall, kh, kw, stride);

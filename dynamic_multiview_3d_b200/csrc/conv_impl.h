@@ -73,7 +73,7 @@ void tc_set_dact(const void* y_bf16, int act);
 bool tc_finish_dact();
 // weight-packing mode of the NEXT tc_* launch of this thread: 0 = pack then run, DMV_ALGO_PACK_ONLY, DMV_ALGO_PREPACKED
 void tc_set_pack_mode(int mode);
-size_t tc_wgrad_workspace(int taps, int Cin, int Cout, long long pixels);
+size_t tc_wgrad_workspace(int taps, int Cin, int Cout, int N, int Hs, int Ws);      // Hs x Ws: the gradient image
 size_t tc_pack_workspace(int taps, int Cin, int Cout);
 int tc_conv_fwd(const void* x, int xdt, const void* w, const float* bias, void* y, int ydt, int B, int H, int W, int Cin, int Cout,
                 int kh, int kw, int stride, int act, void* ws, size_t ws_bytes, cudaStream_t st);

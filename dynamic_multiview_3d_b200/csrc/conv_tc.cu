@@ -861,6 +861,7 @@ int launch_igemm(const Problem& q, IgemmParams& p, void* workspace, size_t ws_by
     if ((p.d2s || p.planes == 2) && !halo_ok) return fail(DMV_E_UNSUPPORTED_SHAPE, "tc: shape not covered by the halo kernel");
     // Deep, spatially small layers (14^2 / 7^2 at 128-256 channels) have fewer M tiles than SMs: cut N into narrower
     // tiles until the launch fills the persistent grid (the A boxes are then re-read per N tile from L2, which is cheap).
+    bool n_split = false;
     if (!halo_ok && q.n_tile == 0 && !p.d2s && p.planes != 2 && !getenv("DMV_NO_NSPLIT")) {
         const int m_tiles = p.num_classes * p.tiles_per_class;
         int nt = p.n_pad;
@@ -868,6 +869,7 @@ int launch_igemm(const Problem& q, IgemmParams& p, void* workspace, size_t ws_by
         if (nt != p.n_pad) {
             p.n_pad = nt;
             p.n_tiles = ceil_div(q.n_real, nt);
+            n_split = true;
         }
     }
 
@@ -962,7 +964,10 @@ int launch_igemm(const Problem& q, IgemmParams& p, void* workspace, size_t ws_by
             return DMV_E_CUDA;
         }
         count_tc_launch();
-        return check_launch("halo_tc");
+        return check_launch(p.d2s == 2 ? "halo_tc (sub-pixel, coalescing epilogue)"
+                            : p.d2s    ? "halo_tc (sub-pixel)"
+                            : p.planes == 2 ? "halo_tc (parity planes)"
+                                            : "halo_tc");
     }
     // ---- split-K (linear layers): fp32 partials into the workspace, finished by splitk_finish_kernel
     void* final_out = p.out;
@@ -1019,7 +1024,7 @@ int launch_igemm(const Problem& q, IgemmParams& p, void* workspace, size_t ws_by
         return DMV_E_CUDA;
     }
     count_tc_launch();
-    int rc_l = check_launch("igemm_tc");
+    int rc_l = check_launch(p.k_splits > 1 ? "igemm_tc (split-K)" : n_split ? "igemm_tc (N-split)" : "igemm_tc");
     if (rc_l) return rc_l;
     if (p.k_splits > 1) {
         const long long mn = (long long)q.N * q.n_real;
@@ -1452,7 +1457,7 @@ size_t tc_thin_workspace(int N, int Hb, int Wb, int Ct, int Cw, int kh, int kw, 
     const size_t P = align256((size_t)N * ph.out * pw.out * Kp * 2);
     const size_t packed = align256((size_t)Cw * Kp * 2);
     const size_t dwt = align256((size_t)Kp * Cw * 4);
-    const size_t parts = tc_wgrad_workspace(1, Kp, Cw, (long long)N * ph.out * pw.out);
+    const size_t parts = tc_wgrad_workspace(1, Kp, Cw, N, ph.out, pw.out);
     return P + packed + dwt + parts + 1024;
 }
 

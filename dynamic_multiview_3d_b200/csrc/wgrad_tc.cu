@@ -1052,9 +1052,11 @@ int run_wgrad(const WProblem& q, void* ws, size_t ws_bytes, cudaStream_t st) {
 
 namespace dmv {
 
-size_t tc_wgrad_workspace(int taps, int Cin, int Cout, long long pixels) {
-    // mirrors plan_wgrad: one fp32 copy of dW per pixel slice (none when a single slice writes dW directly)
-    if (!wgrad_eligible(Cin, Cout, taps)) return 0;
+size_t tc_wgrad_workspace(int taps, int Cin, int Cout, int N, int Hs, int Ws) {
+    // one fp32 copy of dW per pixel slice (none when a single slice writes dW directly).  The estimate from the pixel
+    // count also covers the halo variants; the generic kernel's own plan is added because its ragged chunk boxes can
+    // outnumber pixels / 16 (e.g. a 15 x 17 gradient image).
+    if (!wgrad_eligible(Cin, Cout, taps) || N <= 0 || Hs <= 0 || Ws <= 0) return 0;
     const int CB = (Cin % 64 == 0) ? 64 : 32;
     const int n_tile = Cout > 256 ? 256 : Cout;
     const int n_tiles = ceil_div(Cout, n_tile);
@@ -1063,10 +1065,16 @@ size_t tc_wgrad_workspace(int taps, int Cin, int Cout, long long pixels) {
     if (tpg > m_tiles) tpg = m_tiles;
     const int base = ceil_div(m_tiles, tpg) * n_tiles;
     long long slices = ceil_div(num_sms(), base);
-    const long long max_chunks = ceil_div_ll(pixels, 16);
+    const long long max_chunks = ceil_div_ll((long long)N * Hs * Ws, 16);
     if (slices > max_chunks) slices = max_chunks;
-    if (slices <= 1) return 0;
-    return (size_t)slices * (size_t)taps * Cin * Cout * sizeof(float) + 256;
+    size_t need = slices > 1 ? (size_t)slices * (size_t)taps * Cin * Cout * sizeof(float) : 0;
+    WProblem q;
+    memset(&q, 0, sizeof(q));
+    q.N = N; q.Hs = Hs; q.Ws = Ws; q.Cb = Cin; q.Cs = Cout; q.kh = taps; q.kw = 1;
+    WgradParams p;
+    const size_t plan = plan_wgrad(q, p);
+    if (plan > need) need = plan;
+    return need ? need + 256 : 0;
 }
 
 int tc_conv_wgrad(const void* x, int xdt, const void* dy, float* dw, float* db, int B, int H, int W, int Cin, int Cout, int kh, int kw,
@@ -1131,7 +1139,7 @@ int tc_thin_wgrad(const void* thin, int thin_dtype, const void* wide, float* dw,
     }
     if (!wgrad_eligible(Kp, Cw, 1)) return fail(DMV_E_UNSUPPORTED_SHAPE, "tc_thin_wgrad: channel counts not covered");
     const size_t Pb = al((size_t)N * ph.out * pw.out * Kp * 2), Db = al((size_t)Kp * Cw * 4);
-    const size_t parts = tc_wgrad_workspace(1, Kp, Cw, (long long)N * ph.out * pw.out);
+    const size_t parts = tc_wgrad_workspace(1, Kp, Cw, N, ph.out, pw.out);
     if (!ws || ws_bytes < Pb + Db + parts || ((uintptr_t)ws & 255)) return fail(DMV_E_WORKSPACE, "tc_thin_wgrad: workspace too small or unaligned");
     uint8_t* base = reinterpret_cast<uint8_t*>(ws);
     int rc = thin_im2col(thin, thin_dtype, base, N, Hb, Wb, Ct, kh, kw, stride, st);

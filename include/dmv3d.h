@@ -76,6 +76,9 @@ const char* dmv_arch(void);                 /* "sm_100a" */
 int dmv_last_error(char* buf, size_t n);    /* copies the thread's last error text */
 long long dmv_launch_count(void);           /* kernels launched by this library so far */
 long long dmv_tc_launch_count(void);        /* of which tcgen05 tensor-core kernels */
+/* successful launches so far whose label (the text of the library's launch check, e.g. "halo_tc", "igemm_tc (split-K)")
+ * equals `what`: tells which kernel form a call took.  Thread-safe; 0 for an unknown label or NULL. */
+long long dmv_launch_count_named(const char* what);
 
 /* ---- bilinear sampler --------------------------------------------------------------- *
  * replaces tf.contrib.resampler.resampler -- tf_utils.py:40-42 (resample_layer) and
