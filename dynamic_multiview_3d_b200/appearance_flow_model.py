@@ -173,7 +173,7 @@ class AppearanceFlowModel(ModelBase):
         self.image0, self.disp, self.image1 = image0, disp, image1
         with use_store(self.store):
             self.flow_field = self.buildModel(image0, F.to_bf16(disp))
-        if not F.warp_loss_supported(image0, self.flow_field) or os.environ.get("DMV_NO_WARP_LOSS"):
+        if not F.warp_loss_supported(image0, self.flow_field, image1) or os.environ.get("DMV_NO_WARP_LOSS"):
             with use_store(self.store):
                 self.gen = flow_resample_layer(image0, self.flow_field, self.grid_order)
             return self.build_loss(image1)

@@ -842,10 +842,21 @@ class _WarpLoss(torch.autograd.Function):
         return None, gflow, None, None, None, None, None, None
 
 
-def warp_loss_supported(data, flow):
-    """Shapes the fused kernel covers (the C ABI returns DMV_E_UNSUPPORTED_SHAPE otherwise)."""
+def _passed_aligned16(t):
+    """The buffer a call passes for ``t`` (``t.contiguous()``) starts on a 16-byte boundary: a contiguous tensor is passed
+    as it is, possibly at an offset into its storage; any other is copied into a fresh allocation."""
+    return not t.is_contiguous() or t.data_ptr() % 16 == 0
+
+
+def warp_loss_supported(data, flow, target=None):
+    """True exactly when dmv_sampler_loss_fused accepts the call ``flow_resample_loss(data, flow, target)`` makes: C in
+    {1,3,4}, W*C and Wout*C multiples of 4, an image-shaped flow (Hout > 1) and 16-byte aligned source, flow and target.
+    The C ABI returns DMV_E_UNSUPPORTED_SHAPE otherwise, so a caller with a view at an offset must take the separate calls.
+    Without ``target`` only the source and the flow are checked: pass the target wherever it is known."""
     Cc, W, Wo = data.shape[-1], data.shape[2], flow.shape[2]
-    return flow.dim() == 4 and flow.shape[1] > 1 and Cc in (1, 3, 4) and (W * Cc) % 4 == 0 and (Wo * Cc) % 4 == 0
+    return (flow.dim() == 4 and data.numel() > 0 and flow.numel() > 0 and flow.shape[1] > 1 and Cc in (1, 3, 4)
+            and (W * Cc) % 4 == 0 and (Wo * Cc) % 4 == 0
+            and all(_passed_aligned16(t) for t in (data, flow, target) if t is not None))
 
 
 def flow_resample_loss(data, flow, target, mode="l2", weights=None, inv_count=None, grid_order="ref_yx", unit_upstream=False):

@@ -266,15 +266,15 @@ FORMS = [
 
 # labels checked by other test files (or by the subprocess cases at the end of this file), with where
 EXEMPT = {
-    "sampler_fwd": "sampler: test_sampler_gpu.py",
-    "sampler_fwd(tma)": "sampler: test_sampler_gpu.py",
-    "sampler_grad_warp": "sampler: test_sampler_gpu.py",
-    "sampler_grad_warp(tma)": "sampler: test_sampler_gpu.py",
-    "sampler_box": "sampler: test_sampler_gpu.py",
-    "sampler_grad_data": "sampler: test_sampler_gpu.py",
-    "sampler_loss_fused": "fused warp loss: test_sampler_gpu.py::test_fused_warp_loss_matches_the_three_separate_calls",
-    "loss_flat": "reconstruction loss: test_layers_gpu.py::test_fused_loss",
-    "loss_fused": "view-fusion loss: test_layers_gpu.py::test_masked_loss_and_view_fusion",
+    "sampler_fwd": "sampler tile kernel: test_sampler_loss_edges_gpu.py (4-byte offset source, C = 16, one-row images)",
+    "sampler_fwd(tma)": "sampler TMA kernel, every window path: test_sampler_loss_edges_gpu.py::test_window_paths_match_the_oracle_and_the_tile_kernel",
+    "sampler_grad_warp": "sampler tile kernel: test_sampler_loss_edges_gpu.py (4-byte offset source, C = 16, one-row images)",
+    "sampler_grad_warp(tma)": "sampler TMA kernel, every window path: test_sampler_loss_edges_gpu.py::test_window_paths_match_the_oracle_and_the_tile_kernel",
+    "sampler_box": "sampler grad_data pre-pass: test_sampler_loss_edges_gpu.py::test_sampler_grad_data_generic_channels, test_sampler_gpu.py",
+    "sampler_grad_data": "sampler grad_data, C in {5, 7, 8} and one-row images: test_sampler_loss_edges_gpu.py, test_sampler_gpu.py",
+    "sampler_loss_fused": "fused warp loss: test_sampler_loss_edges_gpu.py::test_fused_warp_loss_edges and the window-path cases",
+    "loss_flat": "reconstruction loss: test_sampler_loss_edges_gpu.py::test_loss_flat_kernel and the block-cap case",
+    "loss_fused": "single-view and view-fusion loss: test_sampler_loss_edges_gpu.py::test_loss_kernel_single_view, test_view_fusion_loss",
     "scale": "upstream loss scalar: test_layers_gpu.py::test_fused_loss",
     "u8_to_f32": "input pipeline: test_layers_gpu.py::test_u8_to_f32_matches_reference_division",
     "u8_crop_resize_bicubic": "input pipeline: test_input_pipeline.py",
