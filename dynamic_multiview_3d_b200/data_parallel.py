@@ -141,6 +141,16 @@ def plan_chunks(var_table, alloc, chunk_elems, world, trainable=None, big=1 << 2
     return chunks, var2chunks, expected
 
 
+def exchange_args(chunks, c, world, shard_end, alloc):
+    """(start, n_slice, slot, replicated) of dmv_dp_exchange_chunk: for chunk ``c`` of ``chunks``, sharded (rank r owns
+    [start + r * n_slice, start + (r + 1) * n_slice)), or for c < 0 the replicated bias tail [shard_end, alloc) in the last
+    slot, its length rounded up to the kernel's multiple of 8."""
+    if c >= 0:
+        s, e = chunks[c]
+        return s, (e - s) // world, c, 0
+    return shard_end, -(-(alloc - shard_end) // 8) * 8, len(chunks), 1
+
+
 class ShardedGradientReducer:
     """ZeRO-1 style exchange: per chunk a reduce-scatter of the gradients (each rank receives the sum of
     its 1/world slice, in place), Adam on the owned slices only (optimizer state and the fp32 masters are
@@ -511,11 +521,7 @@ class FusedShardedReducer(ShardedGradientReducer):
     def _exchange(self, c, st):
         from . import functional as F
         ad, px, f = self.adam, self.px, self.flat
-        if c >= 0:
-            s, e = self.chunks[c]
-            start, n, slot, rep = s, (e - s) // self.world, c, 0
-        else:
-            start, n, slot, rep = self.shard_end, -(-(self.store.alloc - self.shard_end) // 8) * 8, len(self.chunks), 1
+        start, n, slot, rep = exchange_args(self.chunks, c, self.world, self.shard_end, self.store.alloc)
         F._tag[0] = "dp_exchange"
         F.call("dmv_dp_exchange_chunk", px.grad_peers, px.half_peers, px.sig_peers, px.grad_mc, px.half_mc,
                f["master"].data_ptr(), f["m"].data_ptr(), f["v"].data_ptr(), px.local.data_ptr(), start, n, self.rank, self.world,

@@ -283,12 +283,12 @@ EXEMPT = {
     "cast_f32_to_bf16": "dtype casts: test_model_gpu.py (every model step)",
     "cast_bf16_to_f32": "dtype casts: test_model_gpu.py (every model step)",
     "set_flag": "graphed-step flags: test_model_gpu.py::test_train_step_decreases_loss_and_graph_replay_matches_eager",
-    "adam_tick": "Adam: test_layers_gpu.py::test_adam_matches_tf_oracle and the update cases below",
-    "adam_multi": "Adam: test_adam_multi_under_its_switches below",
-    "adam_scalar": "Adam: test_adam_multi_under_its_switches below (odd sizes, 4-byte offset)",
-    "linear_wgrad_adam": "fused FC update: test_fc_update_under_its_switches below",
-    "linear_wgrad_adam (stream)": "fused FC update: test_fc_update_under_its_switches below",
-    "dp_exchange_chunk": "data-parallel exchange: test_dp_gpu.py",
+    "adam_tick": "Adam step scalars to t = 100000: test_update_kernels_gpu.py::test_adam_tick_long_horizon",
+    "adam_multi": "Adam value edges, bit-identical across forms: test_update_kernels_gpu.py; switches: test_adam_multi_under_its_switches below",
+    "adam_scalar": "Adam scalar kernel (4-byte offset, n % 4 = 3 tail): test_update_kernels_gpu.py::test_adam_edges_bit_identical_across_implementations",
+    "linear_wgrad_adam": "fused FC update, generic: test_update_kernels_gpu.py::test_adam_edges_bit_identical_across_implementations; switches below",
+    "linear_wgrad_adam (stream)": "fused FC update, streaming: test_update_kernels_gpu.py::test_adam_edges_bit_identical_across_implementations; switches below",
+    "dp_exchange_chunk": "data-parallel exchange on emulated ranks at its edges, refusals: test_update_kernels_gpu.py; test_dp_gpu.py",
 }
 
 
