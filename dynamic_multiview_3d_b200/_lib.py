@@ -28,6 +28,7 @@ SIGNATURES = {
     "dmv_tc_launch_count": (_ll, []),
     "dmv_launch_count_named": (_ll, [C.c_char_p]),
     "dmv_sampler_fwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _u, _vp]),
+    "dmv_sampler_fwd_shared_src": (_i, [_vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _u, _vp]),
     "dmv_sampler_bwd_workspace_size": (_sz, [_i, _i, _i, _i, _i, _i]),
     "dmv_sampler_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _u, _vp, _sz, _vp]),
     "dmv_sampler_loss_workspace_size": (_sz, [_i, _i, _i]),

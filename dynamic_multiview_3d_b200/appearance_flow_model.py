@@ -95,11 +95,16 @@ class AppearanceFlowModel(ModelBase):
         return lambda: br.join(code)
 
     def buildModel(self, image0, disp):
-        """appearance_flow_model.py:83-127 with the shape rule; activations fused into the layers."""
+        """appearance_flow_model.py:83-127 with the shape rule; activations fused into the layers.  The viewpoint branch
+        is forked before the encoder is enqueued."""
+        viewpoint_code = self._viewpoint_fork(disp)
+        return self._decode(self.encode(image0), viewpoint_code)
+
+    def encode(self, image0):
+        """The image side: e0 .. e4_0 and fc1 -> features [B, 4096] bf16."""
         B, H = image0.shape[0], image0.shape[1]
         h5 = H // 32
         a, g = self.ACT, self.algo
-        viewpoint_code = self._viewpoint_fork(disp)
         e0 = conv2d_msra(image0, 32, 5, 5, 2, 2, "e0", act=a, algo=g)
         e0_0 = conv2d_msra(e0, 32, 5, 5, 1, 1, "e0_0", act=a, algo=g)
         e1 = conv2d_msra(e0_0, 32, 5, 5, 2, 2, "e1", act=a, algo=g)
@@ -111,8 +116,17 @@ class AppearanceFlowModel(ModelBase):
         e4 = conv2d_msra(e3_0, 256, 3, 3, 2, 2, "e4", act=a, algo=g)
         e4_0 = conv2d_msra(e4, 256, 3, 3, 1, 1, "e4_0", act=a, algo=g)
         e4r = F.reshape(e4_0, (B, h5 * h5 * 256))                       # NHWC flatten, (h, w, c) order
-        e5 = linear_msra(e4r, 4096, "fc1", act=a, algo=g)
+        return linear_msra(e4r, 4096, "fc1", act=a, algo=g)
 
+    def decode(self, features, viewpoint):
+        """features [N, 4096] (encode), viewpoint [N, viewpoint_dim] bf16 -> flow field [N, H, H, 2] fp32: the viewpoint
+        code, the joint FCs, the decoder and the flow head."""
+        return self._decode(features, self._viewpoint_fork(viewpoint))
+
+    def _decode(self, e5, viewpoint_code):
+        B, H = e5.shape[0], self.image_shape[0]
+        h5 = H // 32
+        a, g = self.ACT, self.algo
         concated = torch.cat([e5, viewpoint_code()], dim=1)
 
         a3 = linear_msra(concated, 4096, "a3", act=a, algo=g)
@@ -185,6 +199,16 @@ class AppearanceFlowModel(ModelBase):
     def step_loss(self, batch):
         return self.forward_and_loss(batch["image0"], batch["image1"], batch["disp"])
 
+    def render_sources(self):
+        return ("image0",)
+
+    def _render_encode(self, sources):
+        return self.encode(sources["image0"])
+
+    def _render_decode(self, sources, features, viewpoint, group):
+        flow = self.decode(features, viewpoint)
+        return {"gen": F.flow_resampler_shared(sources["image0"], flow, group, self.grid_order), "flow": flow}
+
     def visualize(self, image0, image1, disp, iter_num=None):
         """appearance_flow_model.py:132-179: output / ground-truth / input grids, the flow image and the
         correspondence probes (visualize.py).  The TF session argument becomes the batch itself."""
@@ -220,15 +244,23 @@ class AppearanceFlowTinghui(AppearanceFlowModel):
     """appearance_flow_tinghui.py:5-49 (Zhou et al.-style lighter net, relu trunk)."""
 
     def buildModel(self, image0, disp):
+        viewpoint_code = self._viewpoint_fork(disp)
+        return self._decode(self.encode(image0), viewpoint_code)
+
+    def encode(self, image0):
+        """e0 .. e4, e_fc0, e_fc1 -> features [B, 2048] bf16."""
         B, H = image0.shape[0], image0.shape[1]
         g = self.algo
-        viewpoint_code = self._viewpoint_fork(disp)
         e = image0
         for name, c in [("e0", 16), ("e1", 32), ("e2", 64), ("e3", 128), ("e4", 256)]:
             e = conv2d_msra(e, c, 3, 3, 2, 2, name, act="relu", algo=g)
         e4r = F.reshape(e, (B, (H // 32) ** 2 * 256))
         e_fc0 = linear_msra(e4r, 2048, "e_fc0", act="relu", algo=g)
-        e_fc1 = linear_msra(e_fc0, 2048, "e_fc1", act="relu", algo=g)
+        return linear_msra(e_fc0, 2048, "e_fc1", act="relu", algo=g)
+
+    def _decode(self, e_fc1, viewpoint_code):
+        B, H = e_fc1.shape[0], self.image_shape[0]
+        g = self.algo
         concated = torch.cat([e_fc1, viewpoint_code()], dim=1)
         d_fc0 = linear_msra(concated, 2048, "a3", act="relu", algo=g)
         d_fc1 = linear_msra(d_fc0, (H // 16) ** 2 * 32, "a4", act="relu", algo=g)

@@ -12,6 +12,8 @@
 //         reconstruction loss and grad_warp into one pass (dmv_sampler_loss_fused);
 //       sampler_tile_kernel (any C <= 16, any alignment, 1-D sample lists): cp.async staging,
 //         predicated taps.
+//     The forward of both forms also serves dmv_sampler_fwd_shared_src, where output sample b reads source image
+//     b / group (one source, many viewpoints): a tile still reads exactly one source image.
 //   grad_data : owner-computes scatter.  One CTA owns a 32x16 SOURCE tile; it visits every
 //     32-pixel warp chunk of the output whose tap box intersects it (two-level box table from a
 //     pre-pass), and each warp accumulates into a warp-private shared-memory copy of the tile.
@@ -68,7 +70,8 @@ constexpr int kStageFloats = SAMPLER_STAGE_KB * 256;   // source window in float
 constexpr int kSrcTileW = 32, kSrcTileH = 16;
 
 struct Geom {
-    int B, H, W, C, Ho, Wo;
+    int B, H, W, C, Ho, Wo;   // B: output samples
+    int group;     // forward: output sample b reads source image b / group (dmv_sampler_fwd_shared_src); 1 elsewhere
     int tw_shift;  // output tile is (1024 >> tw_shift) rows x (1 << tw_shift) cols
     int tiles_x, tiles_y;
     unsigned flags;
@@ -147,11 +150,15 @@ __global__ void __launch_bounds__(kThreads, SAMPLER_MINBLOCKS) sampler_tile_kern
     float* __restrict__ out, int32_t* __restrict__ dbg_idx, uint8_t* __restrict__ dbg_mask, Geom g) {
     extern __shared__ float s_win[];
     __shared__ int s_box[4];
+    __shared__ int s_row0;
     const int C = CT ? CT : g.C;
     const int tid = threadIdx.x;
     int b, i0, j0;
     tile_origin(g, blockIdx.x, b, i0, j0);
     if (tid < 4) s_box[tid] = (tid & 1) ? -0x7fffffff : 0x7fffffff;
+    // first source row of the tile's image: b / group with a shared source (forward), else b.  Kept in shared memory and
+    // read where it is used: one more live register costs this kernel spills at its 48-register bound.
+    if (tid == 0) s_row0 = (MODE == 0 ? b / g.group : b) * g.H;
     __syncthreads();
 
     Sample smp[kPPT];
@@ -207,8 +214,9 @@ __global__ void __launch_bounds__(kThreads, SAMPLER_MINBLOCKS) sampler_tile_kern
     const bool staged = any_valid && ((long long)ny * pitch <= kStageFloats);
     if (staged) {
         const int warp = tid >> 5, lane = tid & 31;
+        const int row0 = s_row0;
         for (int r = warp; r < ny; r += kWarps) {
-            const float* src = data + ((long long)b * g.H + ymin + r) * g.W * C + a0;
+            const float* src = data + ((long long)row0 + ymin + r) * g.W * C + a0;
             float* dst = s_win + r * pitch;
 #if SAMPLER_CPASYNC == 16
             if (vec16) { for (int e = lane * 4; e < seg; e += 128) cp_async16(dst + e, src + e); }
@@ -262,7 +270,7 @@ __global__ void __launch_bounds__(kThreads, SAMPLER_MINBLOCKS) sampler_tile_kern
             o_cc = o_fc + C;
         } else {
             base = data;
-            o_ff = (((long long)b * g.H + fy) * g.W + fx) * C;
+            o_ff = (((long long)s_row0 + fy) * g.W + fx) * C;
             o_cf = o_ff + C;
             o_fc = o_ff + (long long)g.W * C;
             o_cc = o_fc + C;
@@ -339,6 +347,7 @@ __global__ void __launch_bounds__(kThreads, (C == 3 && MODE == 0) ? SAMPLER_TMA_
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     int b, i0, j0;
     tile_origin(g, blockIdx.x, b, i0, j0);
+    const int bs = MODE == 0 ? b / g.group : b;    // source image of the tile
     if (tid < 4) s_box[tid] = (tid & 1) ? -0x7fffffff : 0x7fffffff;
     if (tid == 0) {
         tc::mbar_init(&s_bar[0], 1);
@@ -407,7 +416,7 @@ __global__ void __launch_bounds__(kThreads, (C == 3 && MODE == 0) ? SAMPLER_TMA_
     if (staged) {
         if (tid == 0) {
             tc::mbar_expect_tx(&s_bar[0], box * box * C * 4);
-            tc::tma_load_3d(s_win, span < kBoxS ? &map_src : &map_src_l, &s_bar[0], xa * C, ylo, b);
+            tc::tma_load_3d(s_win, span < kBoxS ? &map_src : &map_src_l, &s_bar[0], xa * C, ylo, bs);
         }
         tc::mbar_wait(&s_bar[0], 0);
     }
@@ -442,7 +451,7 @@ __global__ void __launch_bounds__(kThreads, (C == 3 && MODE == 0) ? SAMPLER_TMA_
             }
         } else {  // tap box larger than the window: predicated gathers from global (L1/L2)
             const bool fxi = fx[k] >= 0, cxi = cx <= g.W - 1, fyi = fy[k] >= 0, cyi = cy <= g.H - 1;
-            const float* base = data + (((long long)b * g.H + fy[k]) * g.W + fx[k]) * C;
+            const float* base = data + (((long long)bs * g.H + fy[k]) * g.W + fx[k]) * C;
             const int rowf = g.W * C;
 #pragma unroll
             for (int c = 0; c < C; ++c) {
@@ -805,6 +814,7 @@ int make_geom(Geom& g, int B, int H, int W, int C, int Ho, int Wo, unsigned flag
     DMV_REQUIRE(C <= 16, DMV_E_UNSUPPORTED_SHAPE, "sampler: C > 16 unsupported");
     DMV_REQUIRE((flags & ~3u) == 0, DMV_E_INVALID_ARG, "sampler: unknown flag");
     g.B = B; g.H = H; g.W = W; g.C = C; g.Ho = Ho; g.Wo = Wo; g.flags = flags;
+    g.group = 1;
     g.tw_shift = (Ho == 1) ? 10 : 5;  // 1-D sample lists use 1x1024 tiles, images 32x32
     g.tiles_x = ceil_div(Wo, 1 << g.tw_shift);
     g.tiles_y = ceil_div(Ho, kTilePix >> g.tw_shift);
@@ -820,9 +830,10 @@ int launch_tile(const float* data, const float* wf, const float* go, float* out,
     if (SAMPLER_TMA && g.tw_shift == 5 && (g.C == 1 || g.C == 3 || g.C == 4) && ((g.W * g.C) & 3) == 0 && ((g.Wo * g.C) & 3) == 0 &&
         aligned && (!di || ((uintptr_t)di & 15) == 0)) {
         CUtensorMap map_src, map_src_l, map_io;
-        int rc = encode_f32_map(&map_src, data, g.W * g.C, g.H, g.B, kBoxS * g.C, kBoxS);
+        const int src_images = g.B / g.group;
+        int rc = encode_f32_map(&map_src, data, g.W * g.C, g.H, src_images, kBoxS * g.C, kBoxS);
         if (rc) return rc;
-        rc = encode_f32_map(&map_src_l, data, g.W * g.C, g.H, g.B, kBoxL * g.C, kBoxL);
+        rc = encode_f32_map(&map_src_l, data, g.W * g.C, g.H, src_images, kBoxL * g.C, kBoxL);
         if (rc) return rc;
         rc = encode_f32_map(&map_io, MODE == 0 ? out : go, g.Wo * g.C, g.Ho, g.B, 32 * g.C, 32);
         if (rc) return rc;
@@ -875,6 +886,19 @@ int dmv_sampler_fwd(const float* data, const float* wf, float* out, int32_t* dbg
     int rc = make_geom(g, B, H, W, C, Hout, Wout, flags);
     if (rc) return rc;
     return launch_tile<0>(data, wf, nullptr, out, dbg_idx, dbg_mask, g, (cudaStream_t)stream);
+}
+
+int dmv_sampler_fwd_shared_src(const float* data, int B_src, int group, const float* wf, float* out, int H, int W, int C,
+                               int Hout, int Wout, unsigned flags, void* stream) {
+    DMV_REQUIRE(data && wf && out, DMV_E_INVALID_ARG, "sampler_fwd_shared_src: null pointer");
+    DMV_REQUIRE(((uintptr_t)wf & 7) == 0, DMV_E_ALIGN, "sampler_fwd_shared_src: warp/flow must be 8-byte aligned");
+    DMV_REQUIRE(B_src > 0 && group > 0, DMV_E_INVALID_ARG, "sampler_fwd_shared_src: non-positive B_src or group");
+    DMV_REQUIRE((long long)B_src * group < (1ll << 31), DMV_E_UNSUPPORTED_SHAPE, "sampler_fwd_shared_src: too many samples");
+    Geom g;
+    int rc = make_geom(g, B_src * group, H, W, C, Hout, Wout, flags);
+    if (rc) return rc;
+    g.group = group;
+    return launch_tile<0>(data, wf, nullptr, out, nullptr, nullptr, g, (cudaStream_t)stream);
 }
 
 size_t dmv_sampler_bwd_workspace_size(int B, int H, int W, int C, int Hout, int Wout) {

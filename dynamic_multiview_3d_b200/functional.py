@@ -302,12 +302,40 @@ def workspace(nbytes, device):
     # keyed by the ROLE of the current stream, not by the stream object: capture streams come and go (one per captured
     # graph) and a buffer per stream object would never be released
     br = _side.get((device.type, device.index, "branch")) if device.type == "cuda" else None
-    key = (device.type, device.index, "branch" if (br is not None and torch.cuda.current_stream(device) == br) else "main")
+    role = "branch" if (br is not None and torch.cuda.current_stream(device) == br) else "main"
+    key = (device.type, device.index, role) if _render_role[0] is None else (device.type, device.index, role, _render_role[0])
     ws = _workspaces.get(key)
     if ws is None or ws.numel() < nbytes:
         ws = torch.empty(max(int(nbytes), 1 << 20), dtype=torch.uint8, device=device)
         _workspaces[key] = ws
     return ws
+
+
+# --- rendering next to training ------------------------------------------------------------------------------------
+# A captured train step holds the addresses of the workspaces and prepack buffers it was captured with.  A render at
+# B x V samples needs larger workspaces; growing the training ones would free memory the graph still uses.  Inside
+# render_scope every workspace is keyed by the scope's role as well, prepacking is off (the layers pack inline) and the
+# FC matrices keep the row count of the training pass (optimizer.fusable reads it).
+_render_role = [None]
+
+
+class render_scope:
+    """Context: launches of an inference pass that must leave every training buffer alone.  ``role`` names the set of
+    workspaces it uses: a captured render graph takes its own so that a later render of another size cannot move them."""
+
+    def __init__(self, role="render"):
+        self.role = role
+
+    def __enter__(self):
+        self.prev = _render_role[0]
+        _render_role[0] = self.role
+
+    def __exit__(self, *a):
+        _render_role[0] = self.prev
+
+
+def rendering():
+    return _render_role[0] is not None
 
 
 # --- weight packing off the critical chain ------------------------------------------------------------------------
@@ -326,7 +354,8 @@ class Prepack(object):
     @staticmethod
     def enabled(store):
         import os
-        return store.device.type == "cuda" and os.environ.get("DMV_PREPACK", "1") == "1" and not _meta_depth[0] and _profile[0] is None
+        return (store.device.type == "cuda" and os.environ.get("DMV_PREPACK", "1") == "1" and not _meta_depth[0] and _profile[0] is None
+                and _render_role[0] is None)
 
     def register(self, key, nbytes, pack_call):
         if key not in self.entries:
@@ -635,10 +664,11 @@ class _Linear(torch.autograd.Function):
         M, K = x.shape
         wk, N = wvar.shape
         assert wk == K, (wvar.name, wvar.shape, x.shape)
-        wvar.rows = M
         y = torch.empty((M, N), dtype=torch.bfloat16, device=x.device)
         _tag[0] = wvar.name
-        if wvar.store.pre_use_hook is not None:
+        if _render_role[0] is None:
+            wvar.rows = M
+        if wvar.store.pre_use_hook is not None and _render_role[0] is None:   # a render flushes pending updates first
             wvar.store.pre_use_hook(wvar)        # a deferred optimizer update of this matrix must have landed
         ws = workspace(_lib.load().dmv_conv_workspace_size(M, 1, 1, K, N, 1, 1, 1), x.device)
         call("dmv_linear_fwd", _p(x), _p(wvar.half), _p(bvar.master) if bvar is not None else None, _p(y), M, K, N, ACT[act],
@@ -802,6 +832,32 @@ def flow_resampler(data, flow, grid_order="ref_yx"):
     if grid_order not in ("ref_yx", "xy"):
         raise ValueError(grid_order)
     return _Resampler.apply(data, flow, flags)
+
+
+def flow_resampler_shared(data, flow, group, grid_order="ref_yx"):
+    """flow_resampler with each source shared by ``group`` consecutive flows: data [B_src,H,W,C], flow [B_src*group,Ho,Wo,2]
+    -> [B_src*group,Ho,Wo,C], output sample n warping data[n // group].  One launch (dmv_sampler_fwd_shared_src), no copy of
+    the sources.  Forward only: it raises where autograd would need a gradient through it."""
+    if grid_order not in ("ref_yx", "xy"):
+        raise ValueError(grid_order)
+    _need_cuda(data, flow)
+    if torch.is_grad_enabled() and (data.requires_grad or flow.requires_grad):
+        raise RuntimeError("flow_resampler_shared has no backward: call it under torch.no_grad() or on tensors that need no gradient")
+    if data.dtype != torch.float32 or flow.dtype != torch.float32:
+        raise TypeError("resampler runs in float32 (reference precision)")
+    if data.dim() != 4 or flow.dim() != 4 or flow.shape[-1] != 2:
+        raise ValueError("data [B_src,H,W,C] and flow [B_src*group,Ho,Wo,2] expected, got %s and %s" % (tuple(data.shape), tuple(flow.shape)))
+    group = int(group)
+    B_src, H, W, Cc = data.shape
+    if flow.shape[0] != B_src * group:
+        raise ValueError("flow holds %d samples, not B_src * group = %d * %d" % (flow.shape[0], B_src, group))
+    data, flow = data.contiguous(), flow.contiguous()
+    Ho, Wo = flow.shape[1], flow.shape[2]
+    out = torch.empty((flow.shape[0], Ho, Wo, Cc), dtype=torch.float32, device=data.device)
+    flags = SAMPLER_ADD_GRID | (SAMPLER_GRID_XY if grid_order == "xy" else 0)
+    _tag[0] = "sampler"
+    call("dmv_sampler_fwd_shared_src", _p(data), B_src, group, _p(flow), _p(out), H, W, Cc, Ho, Wo, flags, _stream(data))
+    return out
 
 
 _loss_wss = {}

@@ -71,8 +71,9 @@ class Base_Prediction_Model(ModelBase):
             e1_0 = conv2d_msra(e1, 32, 5, 5, 1, 1, "e1_0", act="lrelu", algo=g)
             return conv2d_msra(e1_0, 64, 5, 5, 2, 2, "e2", act="lrelu", algo=g)
 
-    def decode(self, x, scope, num_channels, src=None):
-        """main_model.py:68-81 (tanh head) or, with head='flow', a 2-channel flow head + warp of ``src``."""
+    def decode_output(self, x, scope, num_channels, warp=None):
+        """main_model.py:68-81 (``decode``: tanh head) or, with head='flow', a 2-channel flow head and ``warp(flow)``, the
+        warp of the output's source modality."""
         g = self.algo
         B, H = x.shape[0], self.image_shape[0]
         h5 = H // 32
@@ -83,14 +84,22 @@ class Base_Prediction_Model(ModelBase):
             d1_0 = conv2d_msra(d1, 32, 5, 5, 1, 1, "d1_0", act="lrelu", algo=g)
             if self.head == "flow":
                 flow = deconv2d_msra(d1_0, [B, H, H, 2], 5, 5, 2, 2, "d0", act=None, algo=g, out_dtype=torch.float32)
-                return flow_resample_layer(src, flow, self.grid_order), flow
+                return warp(flow), flow
             gen = deconv2d_msra(d1_0, [B, H, H, num_channels], 5, 5, 2, 2, "d0", act="tanh", algo=g, out_dtype=torch.float32)
             return gen, None
 
     def buildModel(self, image0, dimage0, disp):
         """main_model.py:83-142"""
+        srcs = {"image0": image0, "depth0": dimage0}
+        out = self.decode(self.encode(image0, dimage0), disp, lambda key, flow: flow_resample_layer(srcs[key], flow, self.grid_order))
+        self.gen_image1, self.flow_image1 = out.get("gen_image1"), out.get("flow_image1")
+        self.gen_dimage1, self.flow_dimage1 = out.get("gen_dimage1"), out.get("flow_dimage1")
+
+    def encode(self, image0, dimage0):
+        """The per-modality pre-encoders, e2_0 .. e4_0 and fc1 -> features [B, 4096] bf16."""
         g = self.algo
-        B, H = image0.shape[0], image0.shape[1]
+        x = image0 if image0 is not None else dimage0
+        B, H = x.shape[0], x.shape[1]
         h5 = H // 32
         concat_list = []
         if self.use_color:
@@ -104,7 +113,15 @@ class Base_Prediction_Model(ModelBase):
         e3_0 = conv2d_msra(e3, 128, 3, 3, 1, 1, "e3_0", act=a, algo=g)
         e4 = conv2d_msra(e3_0, 256, 3, 3, 2, 2, "e4", act=a, algo=g)
         e4_0 = conv2d_msra(e4, 256, 3, 3, 1, 1, "e4_0", act=a, algo=g)
-        e5 = linear_msra(F.reshape(e4_0, (B, h5 * h5 * 256)), 4096, "fc1", act=a, algo=g)
+        return linear_msra(F.reshape(e4_0, (B, h5 * h5 * 256)), 4096, "fc1", act=a, algo=g)
+
+    def decode(self, e5, disp, warp=None):
+        """features [N, 4096] (encode), disp [N, viewpoint_dim] bf16 -> {gen_image1, gen_dimage1} [N, H, H, C] and, with
+        head='flow', {flow_image1, flow_dimage1}: the viewpoint FCs, the joint FCs, the decoder and the heads.
+        ``warp(source_key, flow)`` warps the source modality ("image0" / "depth0") of a flow head."""
+        g, a = self.algo, "lrelu"
+        B, H = e5.shape[0], self.image_shape[0]
+        h5 = H // 32
         a0 = linear_msra(disp, 64, "a0", act=a, algo=g)
         a1 = linear_msra(a0, 64, "a1", act=a, algo=g)
         a2 = linear_msra(a1, 64, "a2", act=a, algo=g)
@@ -118,12 +135,13 @@ class Base_Prediction_Model(ModelBase):
         num_decode = int(self.use_color) + int(self.use_depth)
         d3_0 = conv2d_msra(d3, 64 * num_decode, 5, 5, 1, 1, "d3_0", act=a, algo=g)
         split_list = list(torch.chunk(d3_0, num_decode, dim=3))
-        self.flow_image1 = self.flow_dimage1 = None
+        out = {}
         if self.use_color:       # split_list.pop(): the colour head takes the LAST channel group (main_model.py:131-133)
-            self.gen_image1, self.flow_image1 = self.decode(split_list.pop(), "dec_image1", 3, image0)
+            out["gen_image1"], out["flow_image1"] = self.decode_output(split_list.pop(), "dec_image1", 3, lambda f: warp("image0", f))
         if self.use_depth:
-            self.gen_dimage1, self.flow_dimage1 = self.decode(split_list.pop(), "dec_dimage1", 1, dimage0)
+            out["gen_dimage1"], out["flow_dimage1"] = self.decode_output(split_list.pop(), "dec_dimage1", 1, lambda f: warp("depth0", f))
         assert split_list == []
+        return {k: v for k, v in out.items() if v is not None}
 
     def forward(self, image0, dimage0, disp):
         """image0 [B,H,H,3], dimage0 [B,H,H,1] fp32 in [0,1], disp [B,V] -> dict(gen_image1, gen_dimage1)."""
@@ -160,3 +178,12 @@ class Base_Prediction_Model(ModelBase):
     def step_loss(self, batch):
         self.forward(batch["image0"], batch["depth0"], batch["disp"])
         return self.build_loss(batch["image1"], batch["depth1"])
+
+    def render_sources(self):
+        return (("image0",) if self.use_color else ()) + (("depth0",) if self.use_depth else ())
+
+    def _render_encode(self, sources):
+        return self.encode(sources.get("image0"), sources.get("depth0"))
+
+    def _render_decode(self, sources, features, viewpoint, group):
+        return self.decode(features, viewpoint, lambda key, flow: F.flow_resampler_shared(sources[key], flow, group, self.grid_order))

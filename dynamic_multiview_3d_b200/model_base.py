@@ -12,6 +12,9 @@ here, so the same contract is:
   state_dict()/load_state_dict()   tf.train.Saver over all global variables incl. the Adam slots (train.py:70-71)
 
 ``train_step`` also accepts the class's positional form (``train_step(image0, image1, disp)`` etc.).
+
+Novel views (the single-view classes): ``render(sources, viewpoints)`` encodes each source once and decodes every
+viewpoint from the same features; ``train.GraphedRender`` is its CUDA-graph form.
 """
 import torch
 
@@ -72,6 +75,44 @@ class ModelBase(object):
         """The validation pass of train.py:128-132 (val_summ_op): loss only, no gradient, no update."""
         with torch.no_grad():
             return self.step_loss(self._as_batch(args)).detach()
+
+    # -- rendering -----------------------------------------------------------------------------------------------------
+    def render_sources(self):
+        """Names of the source inputs ``render`` takes."""
+        raise NotImplementedError("%s does not implement render()" % type(self).__name__)
+
+    def render(self, sources, viewpoints):
+        """Novel views of each source.  ``sources``: dict name -> [B, ...] fp32 (``render_sources()``: image0, and depth0
+        for the depth models); ``viewpoints``: [B, V, viewpoint_dim], or [V, viewpoint_dim] for every source.  The
+        encoder runs once per source (batch B), the decoder once per view (batch B * V), and each warp reads its source
+        in place (functional.flow_resampler_shared).  Returns a dict of [B, V, H, W, C] fp32: gen and flow for the flow
+        models; gen_image1 / gen_dimage1 (and flow_image1 / flow_dimage1 with head='flow') for Base_Prediction_Model.
+        Inference only (no_grad); reads no training state and leaves every training buffer where it is."""
+        self.flush_updates()
+        return self._render(sources, viewpoints)
+
+    def _render(self, sources, viewpoints, role="render"):
+        keys = self.render_sources()
+        missing = [k for k in keys if k not in sources]
+        if missing:
+            raise KeyError("%s.render needs sources %s (missing %s)" % (type(self).__name__, keys, missing))
+        B = int(sources[keys[0]].shape[0])
+        if any(int(sources[k].shape[0]) != B for k in keys):
+            raise ValueError("sources differ in batch size: %s" % {k: tuple(sources[k].shape) for k in keys})
+        vp = viewpoints
+        if vp.dim() == 2:
+            vp = vp.unsqueeze(0).expand(B, vp.shape[0], vp.shape[1])
+        if vp.dim() != 3 or vp.shape[0] != B or vp.shape[2] != self.viewpoint_dim:
+            raise ValueError("viewpoints must be [B, V, %d] or [V, %d] with B = %d, got %s"
+                             % (self.viewpoint_dim, self.viewpoint_dim, B, tuple(viewpoints.shape)))
+        V = int(vp.shape[1])
+        from . import functional as F
+        from .variables import use_store
+        with torch.no_grad(), F.render_scope(role), use_store(self.store):
+            self.store._pass_uses = set()           # a fresh pass over the variables (VariableStore.get)
+            feats = self._render_encode(sources).repeat_interleave(V, dim=0)
+            out = self._render_decode(sources, feats, F.to_bf16(vp.reshape(B * V, self.viewpoint_dim)), V)
+        return {k: v.reshape((B, V) + tuple(v.shape[1:])) for k, v in out.items()}
 
     def visualize(self, *a, **k):
         raise NotImplementedError("%s has no visualize(); the reference's own is broken for this class (SURVEY 3.3)" % type(self).__name__)

@@ -97,6 +97,11 @@ class MultiObjectAppFlow(ModelBase):
         self.forward(batch)
         return self.build_loss(batch)
 
+    def render(self, sources, viewpoints):
+        raise NotImplementedError(
+            "MultiObjectAppFlow has no render(): its encoder takes the image, the depth and the object masks of a scene of "
+            "several objects and its heads predict per-object outputs, so a view is not a warp of one source image")
+
     def visualize(self, *args, **kw):
         """multiobject_appflow.py:289-393: imgdata.pkl with every clipped input / output (+ PNG panels)."""
         from .visualize import visualize_multiobject
@@ -234,6 +239,11 @@ class MultiViewFusionAppFlow(MultiObjectAppFlow):
     """BASELINE config 5: ``num_views`` source frames per sample on the multi-object trunk, one 3-channel
     flow + confidence head per frame, softmax fusion (module docstring)."""
     SRC_KEYS = ("image0", "depth0", "image0_mask0", "image0_mask1")
+
+    def render(self, sources, viewpoints):
+        raise NotImplementedError(
+            "MultiViewFusionAppFlow has no render(): each view it predicts fuses the warps of num_views source frames of "
+            "a multi-object scene by predicted confidences, and rendering covers one source image per sample")
 
     def __init__(self, conf, load_tfrec=True, build_loss=True, device=None):
         self.num_views = int(conf.get("num_views", 4))

@@ -176,6 +176,59 @@ class GraphedTrainStep:
         return LossFuture(slot, ev)
 
 
+class GraphedRender:
+    """model.render for B sources x V viewpoints captured once into a CUDA graph and replayed.  Sources and viewpoints
+    are copied into static device buffers (``sources``: dict of [B, H, W, C]; ``viewpoints``: [B, V, viewpoint_dim]) before
+    each replay; the result is a dict of static [B, V, H, W, C] tensors that the next replay overwrites.  The graph reads
+    the parameters and writes only its own buffers: its workspaces are its own (functional.render_scope), so a captured
+    train step and eager renders of other sizes can run in the same process."""
+
+    def __init__(self, model, B, V, warmup=2):
+        self.model, self.B, self.V, self.warmup = model, int(B), int(V), warmup
+        dev, H = model.device, model.image_shape[0]
+        chans = {"image0": 3, "depth0": 1}
+        self.sources = {k: torch.zeros((self.B, H, H, chans[k]), dtype=torch.float32, device=dev) for k in model.render_sources()}
+        self.viewpoints = torch.zeros((self.B, self.V, model.viewpoint_dim), dtype=torch.float32, device=dev)
+        self.role = "graph%d" % id(self)
+        self.graph = None
+        self.out = None
+
+    def capture(self):
+        m = self.model
+        m.flush_updates()
+        main = torch.cuda.current_stream(m.device)
+        side = torch.cuda.Stream(device=m.device)
+        side.wait_stream(main)
+        with torch.cuda.stream(side):
+            for _ in range(self.warmup):          # workspaces grow and modules load outside the capture
+                m._render(self.sources, self.viewpoints, role=self.role)
+        main.wait_stream(side)
+        torch.cuda.synchronize(m.device)
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.graph, stream=side):
+            self.out = m._render(self.sources, self.viewpoints, role=self.role)
+        torch.cuda.synchronize(m.device)
+        return self
+
+    def __call__(self, sources=None, viewpoints=None):
+        """Copy in ``sources`` (fp32, or uint8 pixels prepared on the device) and ``viewpoints`` ([B, V, d] or [V, d]) when
+        given, then replay.  Parameters changed by training since the last call are picked up (pending updates flushed)."""
+        from . import functional as F
+        for k, src in (sources or {}).items():
+            dst = self.sources[k]
+            if src.dtype == torch.uint8:
+                F.prepare_images(src.to(dst.device, non_blocking=True), dst.shape[-2], out=dst)
+            else:
+                dst.copy_(src, non_blocking=True)
+        if viewpoints is not None:
+            self.viewpoints.copy_(viewpoints.expand(self.viewpoints.shape) if viewpoints.dim() == 2 else viewpoints, non_blocking=True)
+        if self.graph is None:
+            self.capture()
+        self.model.flush_updates()
+        self.graph.replay()
+        return self.out
+
+
 class LossFuture(object):
     def __init__(self, slot, event):
         self.slot, self.event = slot, event

@@ -94,6 +94,15 @@ int dmv_sampler_fwd(const float* data, const float* wf, float* out, int32_t* dbg
                     uint8_t* dbg_mask, int B, int H, int W, int C, int Hout, int Wout,
                     unsigned flags, void* stream);
 
+/* dmv_sampler_fwd with a source shared by `group` consecutive output samples (rendering one source image from many
+ * viewpoints without copying it):
+ *   data [B_src,H,W,C] f32      wf [B_src*group,Hout,Wout,2] f32      out [B_src*group,Hout,Wout,C] f32
+ * out sample n (0 <= n < B_src*group) samples data[n / group]; every value has the bits dmv_sampler_fwd gives on the
+ * source repeated `group` times along the batch.  No debug outputs; no backward (inference only).
+ * DMV_E_INVALID_ARG / DMV_E_UNSUPPORTED_SHAPE / DMV_E_ALIGN as dmv_sampler_fwd; a refused call launches nothing. */
+int dmv_sampler_fwd_shared_src(const float* data, int B_src, int group, const float* wf, float* out,
+                               int H, int W, int C, int Hout, int Wout, unsigned flags, void* stream);
+
 /* replaces the registered gradient "ResamplerGrad" (implicit via
  * tf.train.AdamOptimizer.minimize, appearance_flow_model.py:77).
  *   grad_data [B,H,W,C] f32 or NULL (skip: the source is a network input)
