@@ -33,6 +33,8 @@ SIGNATURES = {
     "dmv_sampler_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _u, _vp, _sz, _vp]),
     "dmv_sampler_loss_workspace_size": (_sz, [_i, _i, _i]),
     "dmv_sampler_loss_fused": (_i, [_vp, _vp, _vp, C.POINTER(_f), _i, _f, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _u, _vp, _sz, _vp]),
+    "dmv_sampler_loss_fused_shared_src": (_i, [_vp, _i, _i, _vp, _vp, C.POINTER(_f), _i, _f, _vp, _vp, _vp, _i, _i, _i, _i, _i, _u, _vp, _sz, _vp]),
+    "dmv_sampler_grad_flow_shared_src": (_i, [_vp, _i, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _u, _vp]),
     "dmv_loss_workspace_size": (_sz, [_ll]),
     "dmv_loss_fused_fwd_bwd": (_i, [_vp, _vp, _i, _vp, _vp, C.POINTER(_f), _i, _f, _vp, _vp, _vp, _vp, _ll, _i, _vp, _sz, _vp]),
     "dmv_scale_by_device_scalar": (_i, [_vp, _vp, _ll, _vp]),
@@ -55,6 +57,7 @@ SIGNATURES = {
     "dmv_act_bwd": (_i, [_vp, _vp, _vp, _i, _ll, _i, _vp]),
     "dmv_act_bwd_bias_workspace_size": (_sz, [_ll, _i]),
     "dmv_act_bwd_bias": (_i, [_vp, _vp, _vp, _vp, _ll, _i, _i, _vp, _sz, _vp]),
+    "dmv_act_bwd_bias_grouped": (_i, [_vp, _ll, _i, _vp, _vp, _vp, _ll, _i, _i, _vp, _sz, _vp]),
     "dmv_cast_f32_to_bf16": (_i, [_vp, _vp, _ll, _vp]),
     "dmv_cast_bf16_to_f32": (_i, [_vp, _vp, _ll, _vp]),
     "dmv_adam_tick": (_i, [_vp, _f, _f, _f, _vp]),

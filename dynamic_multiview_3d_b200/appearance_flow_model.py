@@ -15,7 +15,12 @@ reproduces the reference shapes and 224 gives BASELINE's.
 
 Extra conf keys (all optional): image_size (128), viewpoint_dim (2), loss ('l2' = reference,
 'l1' = north-star), grid_order ('ref_yx' = the reference's transposing (Y,X) grid, 'xy'),
-algo ('auto'|'simt'|'tcgen05'), seed (0).
+algo ('auto'|'simt'|'tcgen05'), seed (0), num_targets (1).
+
+Several targets per source: a batch with disp [B, T, viewpoint_dim] and image1 [B, T, H, H, 3] trains B sources x T
+targets.  The encoder runs once per source, fc1 / e_fc1 hands each source's features to its T targets
+(functional.linear(group=T)), the decoder runs at B*T rows and the warp reads each source in place.  The loss is the
+mean over all B*T target images.  conf['num_targets'] only shapes input_spec(); batch_size is the number of sources.
 """
 import os
 
@@ -40,6 +45,9 @@ class AppearanceFlowModel(ModelBase):
             raise ValueError("image_size must be a multiple of 32")
         self.image_shape = [H, H, 3]
         self.viewpoint_dim = int(conf.get("viewpoint_dim", 2))
+        self.num_targets = int(conf.get("num_targets", 1))
+        if self.num_targets < 1:
+            raise ValueError("num_targets must be >= 1")
         self.loss_mode = conf.get("loss", "l2")
         self.grid_order = conf.get("grid_order", "ref_yx")
         self.algo = conf.get("algo", None)
@@ -72,7 +80,9 @@ class AppearanceFlowModel(ModelBase):
 
     def input_spec(self):
         B = self.batch_size
-        return {"image0": tuple([B] + self.image_shape), "image1": tuple([B] + self.image_shape), "disp": (B, self.viewpoint_dim)}
+        T = () if self.num_targets == 1 else (self.num_targets,)
+        return {"image0": tuple([B] + self.image_shape), "image1": tuple([B] + list(T) + self.image_shape),
+                "disp": (B,) + T + (self.viewpoint_dim,)}
 
     # dead variables of the high-dim viewpoint encoder receive no gradient (TF skips None grads)
     def _trainable(self, name):
@@ -94,14 +104,15 @@ class AppearanceFlowModel(ModelBase):
             code = self.decodeAngle(disp)
         return lambda: br.join(code)
 
-    def buildModel(self, image0, disp):
+    def buildModel(self, image0, disp, group=1):
         """appearance_flow_model.py:83-127 with the shape rule; activations fused into the layers.  The viewpoint branch
-        is forked before the encoder is enqueued."""
+        is forked before the encoder is enqueued.  group > 1: disp holds ``group`` consecutive viewpoints per source."""
         viewpoint_code = self._viewpoint_fork(disp)
-        return self._decode(self.encode(image0), viewpoint_code)
+        return self._decode(self.encode(image0, group), viewpoint_code)
 
-    def encode(self, image0):
-        """The image side: e0 .. e4_0 and fc1 -> features [B, 4096] bf16."""
+    def encode(self, image0, group=1):
+        """The image side: e0 .. e4_0 and fc1 -> features [B * group, 4096] bf16 (each source's row repeated ``group``
+        times)."""
         B, H = image0.shape[0], image0.shape[1]
         h5 = H // 32
         a, g = self.ACT, self.algo
@@ -116,7 +127,7 @@ class AppearanceFlowModel(ModelBase):
         e4 = conv2d_msra(e3_0, 256, 3, 3, 2, 2, "e4", act=a, algo=g)
         e4_0 = conv2d_msra(e4, 256, 3, 3, 1, 1, "e4_0", act=a, algo=g)
         e4r = F.reshape(e4_0, (B, h5 * h5 * 256))                       # NHWC flatten, (h, w, c) order
-        return linear_msra(e4r, 4096, "fc1", act=a, algo=g)
+        return linear_msra(e4r, 4096, "fc1", act=a, algo=g, group=group)
 
     def decode(self, features, viewpoint):
         """features [N, 4096] (encode), viewpoint [N, viewpoint_dim] bf16 -> flow field [N, H, H, 2] fp32: the viewpoint
@@ -149,20 +160,34 @@ class AppearanceFlowModel(ModelBase):
     def forward(self, image0, disp, keep=None):
         """image0 [B,H,H,3] fp32 in [0,1], disp [B,V] fp32 -> dict(flow_field, gen); sets the
         reference's attribute names.  warp_pts is formed inside the sampler; read
-        ``self.warp_pts`` to materialise it."""
+        ``self.warp_pts`` to materialise it.  disp [B,T,V]: T targets per source, outputs [B,T,...]."""
         # drop the previous step's tape before building the next one (see VariableStore.new_anchor)
         self.flow_field = self.gen = self.loss = None
         self.store.new_anchor()
         self.image0, self.disp = image0, disp
+        if disp.dim() == 3:
+            with use_store(self.store):
+                flow, T = self._grouped_flow(image0, disp)
+                gen = F.flow_resampler_grouped(image0, flow, T, self.grid_order)
+            self.flow_field, self.gen = _per_source(flow, T), _per_source(gen, T)
+            return {"flow_field": self.flow_field, "gen": self.gen}
         with use_store(self.store):
             self.flow_field = self.buildModel(image0, F.to_bf16(disp))
             self.gen = flow_resample_layer(image0, self.flow_field, self.grid_order)
         return {"flow_field": self.flow_field, "gen": self.gen}
 
+    def _grouped_flow(self, image0, disp):
+        """disp [B, T, V] -> (flow [B*T, H, H, 2], T): each source encoded once, decoded at its T viewpoints."""
+        B, T = int(disp.shape[0]), int(disp.shape[1])
+        if image0.shape[0] != B:
+            raise ValueError("image0 holds %d sources, disp %d" % (image0.shape[0], B))
+        return self.buildModel(image0, F.to_bf16(disp.reshape(B * T, disp.shape[2])), T), T
+
     @property
     def warp_pts(self):
         """warp_pts_layer(flow_field) (appearance_flow_model.py:126), materialised on demand."""
         f = self.flow_field.detach()
+        f = f.reshape((-1,) + tuple(f.shape[-3:]))
         if self.grid_order == "ref_yx":
             return warp_pts_layer(f)
         return f + coords(f.shape[1], f.shape[2], f.shape[0], f.device).flip(-1)
@@ -171,7 +196,7 @@ class AppearanceFlowModel(ModelBase):
         """appearance_flow_model.py:68-73: euclidean_loss(gen, image1) (conf['loss']='l1' for L1).
         The mean runs over the GLOBAL batch under data parallelism."""
         self.image1 = image1
-        n = image1.shape[0] * image1.shape[1] * image1.shape[2] * self.world_size
+        n = image1.numel() // image1.shape[-1] * self.world_size       # every target pixel: B*H*W (B*T*H*W with T targets)
         self.loss = F.reconstruction_loss(self.gen, image1, self.loss_mode, inv_count=1.0 / n, unit_upstream=True)
         return self.loss
 
@@ -182,6 +207,8 @@ class AppearanceFlowModel(ModelBase):
                 or self.device.type == "meta":
             self.forward(image0, disp)
             return self.build_loss(image1)
+        if disp.dim() == 3:
+            return self._grouped_forward_and_loss(image0, image1, disp)
         self.flow_field = self.gen = self.loss = None
         self.store.new_anchor()
         self.image0, self.disp, self.image1 = image0, disp, image1
@@ -194,6 +221,25 @@ class AppearanceFlowModel(ModelBase):
         n = image1.shape[0] * image1.shape[1] * image1.shape[2] * self.world_size
         self.loss, self.gen = F.flow_resample_loss(image0, self.flow_field, image1, self.loss_mode, inv_count=1.0 / n,
                                                    grid_order=self.grid_order, unit_upstream=True)
+        return self.loss
+
+    def _grouped_forward_and_loss(self, image0, image1, disp):
+        """forward_and_loss with T targets per source (image1 [B,T,H,H,3], disp [B,T,V]): the warp of each source by its T
+        flows, the loss over all B*T targets and the flow gradient in one kernel (dmv_sampler_loss_fused_shared_src)."""
+        self.flow_field = self.gen = self.loss = None
+        self.store.new_anchor()
+        self.image0, self.disp, self.image1 = image0, disp, image1
+        with use_store(self.store):
+            flow, T = self._grouped_flow(image0, disp)
+        target = image1.reshape((flow.shape[0],) + tuple(image1.shape[2:]))
+        if not F.warp_loss_supported(image0, flow, target) or os.environ.get("DMV_NO_WARP_LOSS"):
+            self.flow_field = _per_source(flow, T)
+            self.gen = _per_source(F.flow_resampler_grouped(image0, flow, T, self.grid_order), T)
+            return self.build_loss(image1)
+        n = target.numel() // target.shape[-1] * self.world_size
+        self.loss, gen = F.flow_resample_loss(image0, flow, target, self.loss_mode, inv_count=1.0 / n, grid_order=self.grid_order,
+                                              unit_upstream=True, group=T)
+        self.flow_field, self.gen = _per_source(flow, T), _per_source(gen, T)
         return self.loss
 
     def step_loss(self, batch):
@@ -213,7 +259,14 @@ class AppearanceFlowModel(ModelBase):
         """appearance_flow_model.py:132-179: output / ground-truth / input grids, the flow image and the
         correspondence probes (visualize.py).  The TF session argument becomes the batch itself."""
         from .visualize import visualize
+        if disp.dim() == 3:                  # several targets per source: each source's first
+            image1, disp = image1[:, 0], disp[:, 0]
         return visualize(self, image0, image1, disp, iter_num)
+
+
+def _per_source(x, T):
+    """[B*T, ...] -> [B, T, ...]"""
+    return x.reshape((x.shape[0] // T, T) + tuple(x.shape[1:]))
 
 
 class AppFlowHighDimAngle(AppearanceFlowModel):
@@ -243,12 +296,12 @@ class AppFlowLowDimAngle(AppearanceFlowModel):
 class AppearanceFlowTinghui(AppearanceFlowModel):
     """appearance_flow_tinghui.py:5-49 (Zhou et al.-style lighter net, relu trunk)."""
 
-    def buildModel(self, image0, disp):
+    def buildModel(self, image0, disp, group=1):
         viewpoint_code = self._viewpoint_fork(disp)
-        return self._decode(self.encode(image0), viewpoint_code)
+        return self._decode(self.encode(image0, group), viewpoint_code)
 
-    def encode(self, image0):
-        """e0 .. e4, e_fc0, e_fc1 -> features [B, 2048] bf16."""
+    def encode(self, image0, group=1):
+        """e0 .. e4, e_fc0, e_fc1 -> features [B * group, 2048] bf16 (each source's row repeated ``group`` times)."""
         B, H = image0.shape[0], image0.shape[1]
         g = self.algo
         e = image0
@@ -256,7 +309,7 @@ class AppearanceFlowTinghui(AppearanceFlowModel):
             e = conv2d_msra(e, c, 3, 3, 2, 2, name, act="relu", algo=g)
         e4r = F.reshape(e, (B, (H // 32) ** 2 * 256))
         e_fc0 = linear_msra(e4r, 2048, "e_fc0", act="relu", algo=g)
-        return linear_msra(e_fc0, 2048, "e_fc1", act="relu", algo=g)
+        return linear_msra(e_fc0, 2048, "e_fc1", act="relu", algo=g, group=group)
 
     def _decode(self, e_fc1, viewpoint_code):
         B, H = e_fc1.shape[0], self.image_shape[0]

@@ -45,6 +45,14 @@ int dmv_act_bwd_bias(const void* dy_bf16, const void* y_bf16, void* dpre_bf16, f
     return act_bwd_bias(dy_bf16, y_bf16, dpre_bf16, db, rows, C, act, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
+int dmv_act_bwd_bias_grouped(const void* dy_bf16, long long ld_dy, int group, const void* y_bf16, void* dpre_bf16, float* db, long long rows,
+                             int C, int act, void* workspace, size_t workspace_bytes, void* stream) {
+    DMV_REQUIRE(dy_bf16 && y_bf16 && dpre_bf16 && db && rows > 0 && C > 0 && group > 0 && ld_dy >= C, DMV_E_INVALID_ARG,
+                "act_bwd_bias_grouped: bad argument");
+    DMV_REQUIRE(rows <= (1ll << 62) / group / ld_dy, DMV_E_UNSUPPORTED_SHAPE, "act_bwd_bias_grouped: dy too large");
+    return act_bwd_bias(dy_bf16, y_bf16, dpre_bf16, db, rows, C, act, workspace, workspace_bytes, (cudaStream_t)stream, group, ld_dy);
+}
+
 size_t dmv_thin_s2d_size(int N, int H, int W, int C_thin, int C_wide, int kh, int kw, int stride) {
     if (N <= 0 || H <= 0 || W <= 0 || C_thin <= 0 || !thin_s2d_eligible(H, W, C_thin, C_wide, kh, kw, stride)) return 0;
     if (thin_mma_eligible(N, H, W, C_thin, C_wide, kh, kw, stride)) return 0;      // single-kernel form: no prep tensor

@@ -12,8 +12,9 @@ namespace dmv {
 int reduce_partials(const float* part, float* out, long long n, int splits, cudaStream_t st);
 size_t simt_wgrad_workspace(int taps, int Cin, int Cout, long long pixels);
 size_t act_bwd_bias_workspace(long long rows, int C);
+// group > 0: the grouped form (dmv_act_bwd_bias_grouped), dy row pitch ld_dy elements; group == 0: the plain form
 int act_bwd_bias(const void* dy, const void* y, void* dpre, float* db, long long rows, int C, int act, void* ws, size_t ws_bytes,
-                 cudaStream_t st);
+                 cudaStream_t st, int group = 0, long long ld_dy = 0);
 int simt_bias_grad(const void* dy_bf16, float* db, long long pixels, int C, void* ws, size_t ws_bytes, cudaStream_t st);
 int simt_conv_fwd(const void* x, int xdt, const void* w, const float* bias, void* y, int ydt, int B, int H, int W, int Cin,
                   int Cout, int kh, int kw, int stride, int act, cudaStream_t st);

@@ -245,9 +245,12 @@ __global__ void __launch_bounds__(256) colsum_kernel(const T* __restrict__ Y, fl
 // CTA = (CGB column groups of 8 channels) x (256/CGB row lanes) over a contiguous row range; grid.x tiles the
 // columns, grid.y the rows.  Four rows are in flight per thread.  CTA partials are summed in grid.y order by
 // reduce_partials (deterministic).
+// GROUPED (dmv_act_bwd_bias_grouped): row r of dy is the fp32 sum, in t order, of dy rows r * group + t (row pitch ld8
+// uint4s); the ungrouped instantiation compiles exactly the plain kernel.
+template <bool GROUPED>
 __global__ void __launch_bounds__(256) act_bwd_bias_kernel(const uint4* __restrict__ dy, const uint4* __restrict__ y, uint4* __restrict__ dpre,
                                                             float* __restrict__ part, long long rows, int C8, int cgb, long long rows_per_cta,
-                                                            int act) {
+                                                            int act, int group, long long ld8) {
     __shared__ float red[256][9];
     float sum[8];
 #pragma unroll
@@ -271,20 +274,75 @@ __global__ void __launch_bounds__(256) act_bwd_bias_kernel(const uint4* __restri
         return o;
     };
     long long r = r0 + rl;
-    for (; r + 3LL * rstep < r1; r += 4LL * rstep) {
-        uint4 a[4], b[4];
+    if constexpr (GROUPED) {
+        struct F8 { float v[8]; };
+        auto gsum = [&](long long row) {          // fp32 sum of the group's dy rows, t = 0 .. group-1 in order
+            const uint4* p = dy + row * group * ld8 + cg;
+            F8 s;
+            uint4 q = __ldg(p);
+            const __nv_bfloat162* pq = reinterpret_cast<const __nv_bfloat162*>(&q);
 #pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const long long i = (r + (long long)u * rstep) * C8 + cg;
-            a[u] = __ldg(dy + i);
-            b[u] = __ldg(y + i);
+            for (int k = 0; k < 4; ++k) {
+                const float2 f = __bfloat1622float2(pq[k]);
+                s.v[2 * k] = f.x;
+                s.v[2 * k + 1] = f.y;
+            }
+            for (int t = 1; t < group; ++t) {
+                q = __ldg(p + t * ld8);
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    const float2 f = __bfloat1622float2(pq[k]);
+                    s.v[2 * k] += f.x;
+                    s.v[2 * k + 1] += f.y;
+                }
+            }
+            return s;
+        };
+        auto onef = [&](const F8& a, const uint4& b) {
+            uint4 o;
+            const __nv_bfloat162* pb = reinterpret_cast<const __nv_bfloat162*>(&b);
+            __nv_bfloat162* po = reinterpret_cast<__nv_bfloat162*>(&o);
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const float2 fb = __bfloat1622float2(pb[k]);
+                po[k] = __floats2bfloat162_rn(a.v[2 * k] * act_grad_from_output(fb.x, act), a.v[2 * k + 1] * act_grad_from_output(fb.y, act));
+                const float2 q = __bfloat1622float2(po[k]);
+                sum[2 * k] += q.x;
+                sum[2 * k + 1] += q.y;
+            }
+            return o;
+        };
+        for (; r + 3LL * rstep < r1; r += 4LL * rstep) {
+            F8 a[4];
+            uint4 b[4];
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                a[u] = gsum(r + (long long)u * rstep);
+                b[u] = __ldg(y + (r + (long long)u * rstep) * C8 + cg);
+            }
+#pragma unroll
+            for (int u = 0; u < 4; ++u) dpre[(r + (long long)u * rstep) * C8 + cg] = onef(a[u], b[u]);
         }
+        for (; r < r1; r += rstep) {
+            const long long i = r * C8 + cg;
+            dpre[i] = onef(gsum(r), __ldg(y + i));
+        }
+    } else {
+        for (; r + 3LL * rstep < r1; r += 4LL * rstep) {
+            uint4 a[4], b[4];
 #pragma unroll
-        for (int u = 0; u < 4; ++u) dpre[(r + (long long)u * rstep) * C8 + cg] = one(a[u], b[u]);
-    }
-    for (; r < r1; r += rstep) {
-        const long long i = r * C8 + cg;
-        dpre[i] = one(__ldg(dy + i), __ldg(y + i));
+            for (int u = 0; u < 4; ++u) {
+                const long long i = (r + (long long)u * rstep) * C8 + cg;
+                a[u] = __ldg(dy + i);
+                b[u] = __ldg(y + i);
+            }
+#pragma unroll
+            for (int u = 0; u < 4; ++u) dpre[(r + (long long)u * rstep) * C8 + cg] = one(a[u], b[u]);
+        }
+        for (; r < r1; r += rstep) {
+            const long long i = r * C8 + cg;
+            dpre[i] = one(__ldg(dy + i), __ldg(y + i));
+        }
     }
     // reduce over the row lanes: shuffles inside the warp (lanes sharing a column group are cgb apart),
     // then across the 8 warps through shared memory, in a fixed order
@@ -408,8 +466,9 @@ size_t act_bwd_bias_workspace(long long rows, int C) {
 }
 
 int act_bwd_bias(const void* dy, const void* y, void* dpre, float* db, long long rows, int C, int act, void* ws, size_t ws_bytes,
-                 cudaStream_t st) {
+                 cudaStream_t st, int group, long long ld_dy) {
     if (C % 8 || (((uintptr_t)dy | (uintptr_t)y | (uintptr_t)dpre) & 15)) return fail(DMV_E_UNSUPPORTED_SHAPE, "act_bwd_bias: need C % 8 == 0, 16-byte alignment");
+    if (group > 0 && ld_dy % 8) return fail(DMV_E_UNSUPPORTED_SHAPE, "act_bwd_bias_grouped: dy rows must be 16-byte aligned (ld_dy % 8 == 0)");
     const int C8 = C / 8;
     int cgb = 64;
     while (cgb > 1 && (C8 % cgb)) cgb >>= 1;          // largest power of two <= 64 dividing C/8
@@ -424,7 +483,11 @@ int act_bwd_bias(const void* dy, const void* y, void* dpre, float* db, long long
     if (!ws || ws_bytes < (size_t)row_ctas * C * sizeof(float)) return fail(DMV_E_WORKSPACE, "act_bwd_bias: workspace too small");
     float* part = reinterpret_cast<float*>(ws);
     dim3 grid(col_blocks, (unsigned)row_ctas);
-    act_bwd_bias_kernel<<<grid, 256, 0, st>>>((const uint4*)dy, (const uint4*)y, (uint4*)dpre, part, rows, C8, cgb, per, act);
+    if (group > 0)
+        act_bwd_bias_kernel<true><<<grid, 256, 0, st>>>((const uint4*)dy, (const uint4*)y, (uint4*)dpre, part, rows, C8, cgb, per, act, group,
+                                                        ld_dy / 8);
+    else
+        act_bwd_bias_kernel<false><<<grid, 256, 0, st>>>((const uint4*)dy, (const uint4*)y, (uint4*)dpre, part, rows, C8, cgb, per, act, 1, C8);
     int rc = check_launch("act_bwd_bias");
     if (rc) return rc;
     return reduce_partials(part, db, C, (int)row_ctas, st);

@@ -12,8 +12,9 @@
 //         reconstruction loss and grad_warp into one pass (dmv_sampler_loss_fused);
 //       sampler_tile_kernel (any C <= 16, any alignment, 1-D sample lists): cp.async staging,
 //         predicated taps.
-//     The forward of both forms also serves dmv_sampler_fwd_shared_src, where output sample b reads source image
-//     b / group (one source, many viewpoints): a tile still reads exactly one source image.
+//     Both forms also serve the shared-source entry points (dmv_sampler_fwd_shared_src, dmv_sampler_grad_flow_shared_src,
+//     dmv_sampler_loss_fused_shared_src), where output sample b reads source image b / group (one source, many
+//     viewpoints): a tile still reads exactly one source image.
 //   grad_data : owner-computes scatter.  One CTA owns a 32x16 SOURCE tile; it visits every
 //     32-pixel warp chunk of the output whose tap box intersects it (two-level box table from a
 //     pre-pass), and each warp accumulates into a warp-private shared-memory copy of the tile.
@@ -71,7 +72,7 @@ constexpr int kSrcTileW = 32, kSrcTileH = 16;
 
 struct Geom {
     int B, H, W, C, Ho, Wo;   // B: output samples
-    int group;     // forward: output sample b reads source image b / group (dmv_sampler_fwd_shared_src); 1 elsewhere
+    int group;     // output sample b reads source image b / group (the *_shared_src entry points); 1 elsewhere
     int tw_shift;  // output tile is (1024 >> tw_shift) rows x (1 << tw_shift) cols
     int tiles_x, tiles_y;
     unsigned flags;
@@ -156,9 +157,9 @@ __global__ void __launch_bounds__(kThreads, SAMPLER_MINBLOCKS) sampler_tile_kern
     int b, i0, j0;
     tile_origin(g, blockIdx.x, b, i0, j0);
     if (tid < 4) s_box[tid] = (tid & 1) ? -0x7fffffff : 0x7fffffff;
-    // first source row of the tile's image: b / group with a shared source (forward), else b.  Kept in shared memory and
+    // first source row of the tile's image: b / group (group = 1 unless the source is shared).  Kept in shared memory and
     // read where it is used: one more live register costs this kernel spills at its 48-register bound.
-    if (tid == 0) s_row0 = (MODE == 0 ? b / g.group : b) * g.H;
+    if (tid == 0) s_row0 = (b / g.group) * g.H;
     __syncthreads();
 
     Sample smp[kPPT];
@@ -347,7 +348,7 @@ __global__ void __launch_bounds__(kThreads, (C == 3 && MODE == 0) ? SAMPLER_TMA_
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     int b, i0, j0;
     tile_origin(g, blockIdx.x, b, i0, j0);
-    const int bs = MODE == 0 ? b / g.group : b;    // source image of the tile
+    const int bs = b / g.group;    // source image of the tile
     if (tid < 4) s_box[tid] = (tid & 1) ? -0x7fffffff : 0x7fffffff;
     if (tid == 0) {
         tc::mbar_init(&s_bar[0], 1);
@@ -954,19 +955,42 @@ int dmv_sampler_bwd(const float* data, const float* wf, const float* grad_out, f
     return DMV_OK;
 }
 
+int dmv_sampler_grad_flow_shared_src(const float* data, int B_src, int group, const float* wf, const float* grad_out, float* grad_wf,
+                                     int H, int W, int C, int Hout, int Wout, unsigned flags, void* stream) {
+    DMV_REQUIRE(data && wf && grad_out && grad_wf, DMV_E_INVALID_ARG, "sampler_grad_flow_shared_src: null pointer");
+    DMV_REQUIRE(((uintptr_t)wf & 7) == 0 && ((uintptr_t)grad_wf & 7) == 0, DMV_E_ALIGN,
+                "sampler_grad_flow_shared_src: warp buffers must be 8-byte aligned");
+    DMV_REQUIRE(B_src > 0 && group > 0, DMV_E_INVALID_ARG, "sampler_grad_flow_shared_src: non-positive B_src or group");
+    DMV_REQUIRE((long long)B_src * group < (1ll << 31), DMV_E_UNSUPPORTED_SHAPE, "sampler_grad_flow_shared_src: too many samples");
+    Geom g;
+    int rc = make_geom(g, B_src * group, H, W, C, Hout, Wout, flags);
+    if (rc) return rc;
+    g.group = group;
+    return launch_tile<1>(data, wf, grad_out, grad_wf, nullptr, nullptr, g, (cudaStream_t)stream);
+}
+
 size_t dmv_sampler_loss_workspace_size(int B, int Hout, int Wout) {
     if (B <= 0 || Hout <= 0 || Wout <= 0) return 0;
     return (size_t)B * ceil_div(Wout, 32) * ceil_div(Hout, 32) * sizeof(double) + 16;
 }
 
-int dmv_sampler_loss_fused(const float* data, const float* wf, const float* target, const float* chan_weight, int mode, float inv_count,
-                           float* gen_out, float* grad_wf, float* loss_out, int B, int H, int W, int C, int Hout, int Wout,
-                           unsigned flags, void* workspace, size_t workspace_bytes, void* stream) {
+}  // extern "C"
+
+namespace {
+
+// dmv_sampler_loss_fused over B_src source images, output sample n warping source n / group (group = 1: the plain call)
+int sampler_loss_fused(const float* data, int B_src, int group, const float* wf, const float* target, const float* chan_weight, int mode,
+                       float inv_count, float* gen_out, float* grad_wf, float* loss_out, int H, int W, int C, int Hout, int Wout,
+                       unsigned flags, void* workspace, size_t workspace_bytes, void* stream) {
     DMV_REQUIRE(data && wf && target && chan_weight && gen_out && grad_wf && loss_out, DMV_E_INVALID_ARG, "sampler_loss_fused: null pointer");
     DMV_REQUIRE(mode == DMV_LOSS_L2 || mode == DMV_LOSS_L1, DMV_E_INVALID_ARG, "sampler_loss_fused: unknown loss mode");
+    DMV_REQUIRE(B_src > 0 && group > 0, DMV_E_INVALID_ARG, "sampler_loss_fused: non-positive B_src or group");
+    DMV_REQUIRE((long long)B_src * group < (1ll << 31), DMV_E_UNSUPPORTED_SHAPE, "sampler_loss_fused: too many samples");
+    const int B = B_src * group;
     Geom g;
     int rc = make_geom(g, B, H, W, C, Hout, Wout, flags);
     if (rc) return rc;
+    g.group = group;
     const bool aligned = (((uintptr_t)data | (uintptr_t)wf | (uintptr_t)target | (uintptr_t)gen_out | (uintptr_t)grad_wf) & 15) == 0;
     if (!(g.tw_shift == 5 && (C == 1 || C == 3 || C == 4) && ((W * C) & 3) == 0 && ((Wout * C) & 3) == 0 && aligned))
         return fail(DMV_E_UNSUPPORTED_SHAPE, "sampler_loss_fused: needs C in {1,3,4}, 16-byte aligned rows and buffers, image-shaped output");
@@ -974,8 +998,8 @@ int dmv_sampler_loss_fused(const float* data, const float* wf, const float* targ
     DMV_REQUIRE(workspace && workspace_bytes >= dmv_sampler_loss_workspace_size(B, Hout, Wout) && ((uintptr_t)workspace & 7) == 0, DMV_E_WORKSPACE,
                 "sampler_loss_fused: workspace too small or unaligned (it must be zeroed once and not shared)");
     CUtensorMap map_src, map_src_l, map_io, map_tgt;
-    rc = encode_f32_map(&map_src, data, W * C, H, B, kBoxS * C, kBoxS);
-    if (!rc) rc = encode_f32_map(&map_src_l, data, W * C, H, B, kBoxL * C, kBoxL);
+    rc = encode_f32_map(&map_src, data, W * C, H, B_src, kBoxS * C, kBoxS);
+    if (!rc) rc = encode_f32_map(&map_src_l, data, W * C, H, B_src, kBoxL * C, kBoxL);
     if (!rc) rc = encode_f32_map(&map_io, gen_out, Wout * C, Hout, B, 32 * C, 32);
     if (!rc) rc = encode_f32_map(&map_tgt, target, Wout * C, Hout, B, 32 * C, 32);
     if (rc) return rc;
@@ -1001,6 +1025,25 @@ int dmv_sampler_loss_fused(const float* data, const float* wf, const float* targ
     else DMV_LAUNCH_FUSED(4);
 #undef DMV_LAUNCH_FUSED
     return check_launch("sampler_loss_fused");
+}
+
+}  // namespace
+
+extern "C" {
+
+int dmv_sampler_loss_fused(const float* data, const float* wf, const float* target, const float* chan_weight, int mode, float inv_count,
+                           float* gen_out, float* grad_wf, float* loss_out, int B, int H, int W, int C, int Hout, int Wout,
+                           unsigned flags, void* workspace, size_t workspace_bytes, void* stream) {
+    return sampler_loss_fused(data, B, 1, wf, target, chan_weight, mode, inv_count, gen_out, grad_wf, loss_out, H, W, C, Hout, Wout, flags,
+                              workspace, workspace_bytes, stream);
+}
+
+int dmv_sampler_loss_fused_shared_src(const float* data, int B_src, int group, const float* wf, const float* target,
+                                      const float* chan_weight, int mode, float inv_count, float* gen_out, float* grad_wf,
+                                      float* loss_out, int H, int W, int C, int Hout, int Wout, unsigned flags, void* workspace,
+                                      size_t workspace_bytes, void* stream) {
+    return sampler_loss_fused(data, B_src, group, wf, target, chan_weight, mode, inv_count, gen_out, grad_wf, loss_out, H, W, C, Hout, Wout,
+                              flags, workspace, workspace_bytes, stream);
 }
 
 }  // extern "C"

@@ -656,7 +656,7 @@ class _Deconv2d(torch.autograd.Function):
 
 class _Linear(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, anchor, x, wvar, bvar, act, algo, in_cell, out_cell):
+    def forward(ctx, anchor, x, wvar, bvar, act, algo, in_cell, out_cell, group):
         _need_cuda(x)
         x = x.contiguous()
         if x.dtype != torch.bfloat16:
@@ -676,6 +676,9 @@ class _Linear(torch.autograd.Function):
         ctx.save_for_backward(x, y)
         ctx.cfg = (wvar, bvar, act, algo)
         ctx.cells = (in_cell, out_cell)
+        ctx.group = group
+        if group > 1:              # every row consumed ``group`` times: the consumer sees the rows repeated
+            return y.repeat_interleave(group, dim=0)
         return y
 
     @staticmethod
@@ -686,10 +689,18 @@ class _Linear(torch.autograd.Function):
         N = wvar.shape[1]
         st = _stream(x)
         _tag[0] = wvar.name
-        dy = dy.contiguous()
+        dy = dy.contiguous() if ctx.group == 1 else _row_pitched(dy, N)
         bias_done = False
         in_cell, out_cell = ctx.cells
-        if out_cell is not None and out_cell.fused:
+        if ctx.group > 1:
+            # the sum over the ``group`` uses of each row, act' and the bias gradient in one pass; dy may be the slice of a
+            # concat's gradient (row pitch > N)
+            dpre = torch.empty_like(y)
+            ws = workspace(_lib.load().dmv_act_bwd_bias_workspace_size(M, N), x.device)
+            call("dmv_act_bwd_bias_grouped", _p(dy), dy.stride(0), ctx.group, _p(y), _p(dpre), _p(bvar.grad), M, N, ACT[act], _p(ws),
+                 ws.numel(), st)
+            bias_done = True
+        elif out_cell is not None and out_cell.fused:
             dpre = dy
         elif bvar is not None and ACT[act] and N % 8 == 0:
             dpre = torch.empty_like(y)
@@ -730,7 +741,15 @@ class _Linear(torch.autograd.Function):
                 if bvar is not None:
                     wvar.store.notify_grad(bvar)
                 wvar.store.notify_grad(wvar)
-        return None, dx, None, None, None, None, None, None
+        return None, dx, None, None, None, None, None, None, None
+
+
+def _row_pitched(dy, N):
+    """dy [R, N] as dmv_act_bwd_bias_grouped reads it: unit column stride, a row pitch >= N that keeps rows 16-byte aligned.
+    A column slice of a wider gradient qualifies as it is; anything else is copied."""
+    if dy.stride(1) == 1 and dy.stride(0) >= N and dy.stride(0) % 8 == 0 and dy.data_ptr() % 16 == 0:
+        return dy
+    return dy.contiguous()
 
 
 def _tagged(y, cell):
@@ -750,9 +769,20 @@ def deconv2d(x, wvar, out_hw, stride, act=None, algo=None, out_dtype=torch.bfloa
                                    _claim_input(x), cell), cell)
 
 
-def linear(x, wvar, bvar, act=None, algo=None):
-    cell = _out_cell(act, torch.bfloat16)
-    return _tagged(_Linear.apply(wvar.store.anchor, x, wvar, bvar, act, _algo(algo), _claim_input(x), cell), cell)
+def linear(x, wvar, bvar, act=None, algo=None, group=1):
+    """x @ W + b with ``act``.  group > 1: the layer runs once on x [rows, K] and returns [rows * group, N], each row
+    repeated ``group`` times (one source feeding ``group`` targets); backward sums the uses of each row in the bias /
+    activation-gradient pass (dmv_act_bwd_bias_grouped) and runs dgrad / wgrad at the layer's own rows."""
+    group = int(group)
+    if group == 1:
+        cell = _out_cell(act, torch.bfloat16)
+        return _tagged(_Linear.apply(wvar.store.anchor, x, wvar, bvar, act, _algo(algo), _claim_input(x), cell, 1), cell)
+    if group < 1:
+        raise ValueError("group must be >= 1, got %d" % group)
+    if bvar is None or not ACT[act] or wvar.shape[1] % 8:
+        raise ValueError("linear(group=%d) needs a bias, an activation and N %% 8 == 0 (%s: act %s, N %d)"
+                         % (group, wvar.name, act, wvar.shape[1]))
+    return _Linear.apply(wvar.store.anchor, x, wvar, bvar, act, _algo(algo), None, None, group)
 
 
 # ----------------------------------------------------------------------------- activations
@@ -860,6 +890,52 @@ def flow_resampler_shared(data, flow, group, grid_order="ref_yx"):
     return out
 
 
+class _GroupedResampler(torch.autograd.Function):
+    """flow -> warped sources, output sample n reading data[n // group]; the gradient wrt the flow only."""
+
+    @staticmethod
+    def forward(ctx, data, flow, group, flags):
+        B_src, H, W, Cc = data.shape
+        Ho, Wo = flow.shape[1], flow.shape[2]
+        out = torch.empty((flow.shape[0], Ho, Wo, Cc), dtype=torch.float32, device=data.device)
+        _tag[0] = "sampler"
+        call("dmv_sampler_fwd_shared_src", _p(data), B_src, group, _p(flow), _p(out), H, W, Cc, Ho, Wo, flags, _stream(data))
+        ctx.save_for_backward(data, flow)
+        ctx.geom = (B_src, group, H, W, Cc, Ho, Wo, flags)
+        return out
+
+    @staticmethod
+    def backward(ctx, go):
+        data, flow = ctx.saved_tensors
+        B_src, group, H, W, Cc, Ho, Wo, flags = ctx.geom
+        go = go.contiguous()
+        gw = torch.empty_like(flow)
+        _tag[0] = "sampler"
+        call("dmv_sampler_grad_flow_shared_src", _p(data), B_src, group, _p(flow), _p(go), _p(gw), H, W, Cc, Ho, Wo, flags, _stream(data))
+        return None, gw, None, None
+
+
+def flow_resampler_grouped(data, flow, group, grid_order="ref_yx"):
+    """Differentiable flow_resampler with each source shared by ``group`` consecutive flows (training on several targets of
+    one source): data [B_src,H,W,C], flow [B_src*group,Ho,Wo,2] -> [B_src*group,Ho,Wo,C], output sample n warping
+    data[n // group].  Backward gives the flow gradient (dmv_sampler_grad_flow_shared_src); the source is a network input
+    and gets none: it raises if ``data`` needs a gradient."""
+    if grid_order not in ("ref_yx", "xy"):
+        raise ValueError(grid_order)
+    _need_cuda(data, flow)
+    if torch.is_grad_enabled() and data.requires_grad:
+        raise RuntimeError("flow_resampler_grouped has no gradient wrt the source: pass a source that needs no gradient")
+    if data.dtype != torch.float32 or flow.dtype != torch.float32:
+        raise TypeError("resampler runs in float32 (reference precision)")
+    if data.dim() != 4 or flow.dim() != 4 or flow.shape[-1] != 2:
+        raise ValueError("data [B_src,H,W,C] and flow [B_src*group,Ho,Wo,2] expected, got %s and %s" % (tuple(data.shape), tuple(flow.shape)))
+    group = int(group)
+    if group < 1 or flow.shape[0] != data.shape[0] * group:
+        raise ValueError("flow holds %d samples, not B_src * group = %d * %d" % (flow.shape[0], data.shape[0], group))
+    flags = SAMPLER_ADD_GRID | (SAMPLER_GRID_XY if grid_order == "xy" else 0)
+    return _GroupedResampler.apply(data.contiguous(), flow.contiguous(), group, flags)
+
+
 _loss_wss = {}
 
 
@@ -868,10 +944,11 @@ class _WarpLoss(torch.autograd.Function):
     d loss / d flow in one kernel (dmv_sampler_loss_fused).  The source and the target are network inputs."""
 
     @staticmethod
-    def forward(ctx, data, flow, target, flags, weights, mode, inv_count, unit_upstream):
+    def forward(ctx, data, flow, target, flags, weights, mode, inv_count, unit_upstream, group):
         _need_cuda(data, flow, target)
         data, flow, target = data.contiguous(), flow.contiguous(), target.contiguous()
-        B, H, W, Cc = data.shape
+        B_src, H, W, Cc = data.shape
+        B = flow.shape[0]
         Ho, Wo = flow.shape[1], flow.shape[2]
         gen = torch.empty((B, Ho, Wo, Cc), dtype=torch.float32, device=data.device)
         gflow = torch.empty_like(flow)
@@ -883,8 +960,12 @@ class _WarpLoss(torch.autograd.Function):
         if ws is None or ws.numel() < nws:             # zeroed once: holds a self-resetting counter
             ws = _loss_wss[key] = torch.zeros(int(nws), dtype=torch.uint8, device=data.device)
         _tag[0] = "warp_loss"
-        call("dmv_sampler_loss_fused", _p(data), _p(flow), _p(target), w, LOSS[mode], float(inv_count), _p(gen), _p(gflow), _p(loss),
-             B, H, W, Cc, Ho, Wo, flags, _p(ws), ws.numel(), _stream(data))
+        if group == 1:
+            call("dmv_sampler_loss_fused", _p(data), _p(flow), _p(target), w, LOSS[mode], float(inv_count), _p(gen), _p(gflow), _p(loss),
+                 B, H, W, Cc, Ho, Wo, flags, _p(ws), ws.numel(), _stream(data))
+        else:
+            call("dmv_sampler_loss_fused_shared_src", _p(data), B_src, group, _p(flow), _p(target), w, LOSS[mode], float(inv_count), _p(gen),
+                 _p(gflow), _p(loss), H, W, Cc, Ho, Wo, flags, _p(ws), ws.numel(), _stream(data))
         ctx.gflow, ctx.unit_upstream = gflow, unit_upstream
         ctx.mark_non_differentiable(gen)
         return loss, gen
@@ -895,7 +976,7 @@ class _WarpLoss(torch.autograd.Function):
         if not ctx.unit_upstream:
             _tag[0] = "warp_loss"
             call("dmv_scale_by_device_scalar", _p(gflow), _p(gloss.contiguous().to(torch.float32)), gflow.numel(), _stream(gflow))
-        return None, gflow, None, None, None, None, None, None
+        return None, gflow, None, None, None, None, None, None, None
 
 
 def _passed_aligned16(t):
@@ -915,9 +996,11 @@ def warp_loss_supported(data, flow, target=None):
             and all(_passed_aligned16(t) for t in (data, flow, target) if t is not None))
 
 
-def flow_resample_loss(data, flow, target, mode="l2", weights=None, inv_count=None, grid_order="ref_yx", unit_upstream=False):
+def flow_resample_loss(data, flow, target, mode="l2", weights=None, inv_count=None, grid_order="ref_yx", unit_upstream=False, group=1):
     """(loss, gen) of the training step's tail: warp ``data`` by ``flow`` (grid formed in the kernel), compare with
-    ``target``.  One launch instead of sampler forward + loss + sampler backward."""
+    ``target``.  One launch instead of sampler forward + loss + sampler backward.  group > 1: ``data`` holds B_src
+    sources and flow / target B_src * group samples, sample n warping source n // group
+    (dmv_sampler_loss_fused_shared_src)."""
     if grid_order not in ("ref_yx", "xy"):
         raise ValueError(grid_order)
     flags = SAMPLER_ADD_GRID | (SAMPLER_GRID_XY if grid_order == "xy" else 0)
@@ -925,7 +1008,10 @@ def flow_resample_loss(data, flow, target, mode="l2", weights=None, inv_count=No
     weights = [1.0] * Cc if weights is None else list(weights)
     if inv_count is None:
         inv_count = 1.0 / (target.numel() // Cc)
-    return _WarpLoss.apply(data, flow, target, flags, tuple(weights), mode, inv_count, unit_upstream)
+    group = int(group)
+    if group < 1 or flow.shape[0] != data.shape[0] * group:
+        raise ValueError("flow holds %d samples, not B_src * group = %d * %d" % (flow.shape[0], data.shape[0], group))
+    return _WarpLoss.apply(data, flow, target, flags, tuple(weights), mode, inv_count, unit_upstream, group)
 
 
 def resampler_debug(data, wf, flags=0):

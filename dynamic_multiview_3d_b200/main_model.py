@@ -11,7 +11,9 @@ Feature switches are key-presence tests on ``conf`` as in the reference (``'use_
 Extensions (optional conf keys): image_size (128), viewpoint_dim (2), loss ('l2' reference | 'l1' per-channel L1,
 tf_utils.py:22), head ('tanh' reference | 'flow': each head emits a 2-channel flow and the output is the bilinear
 warp of its source modality -- the north-star's "warped RGB/depth"; precedent: multiobject_appflow.py:191-209),
-grid_order, algo, seed.  The reference ignores conf['batch_size'] (main_model.py:19 hard-codes 64); here conf wins.
+grid_order, algo, seed, num_targets (1).  The reference ignores conf['batch_size'] (main_model.py:19 hard-codes 64); here
+conf wins.  Several targets per source (disp [B, T, V], image1 / depth1 [B, T, H, H, C]) train as the appearance-flow
+models do (appearance_flow_model.py): one encoding per source, B*T decoded targets, the loss over all of them.
 """
 import torch
 
@@ -35,6 +37,9 @@ class Base_Prediction_Model(ModelBase):
         self.viewpoint_dim = int(conf.get("viewpoint_dim", 2))
         self.loss_mode = conf.get("loss", "l2")
         self.head = conf.get("head", "tanh")
+        self.num_targets = int(conf.get("num_targets", 1))
+        if self.num_targets < 1:
+            raise ValueError("num_targets must be >= 1")
         self.grid_order = conf.get("grid_order", "ref_yx")
         self.algo = conf.get("algo", None)
         self.use_color = "use_color" in conf
@@ -88,15 +93,20 @@ class Base_Prediction_Model(ModelBase):
             gen = deconv2d_msra(d1_0, [B, H, H, num_channels], 5, 5, 2, 2, "d0", act="tanh", algo=g, out_dtype=torch.float32)
             return gen, None
 
-    def buildModel(self, image0, dimage0, disp):
-        """main_model.py:83-142"""
+    def buildModel(self, image0, dimage0, disp, group=1):
+        """main_model.py:83-142.  group > 1: disp holds ``group`` consecutive viewpoints per source."""
         srcs = {"image0": image0, "depth0": dimage0}
-        out = self.decode(self.encode(image0, dimage0), disp, lambda key, flow: flow_resample_layer(srcs[key], flow, self.grid_order))
+        if group == 1:
+            warp = lambda key, flow: flow_resample_layer(srcs[key], flow, self.grid_order)
+        else:
+            warp = lambda key, flow: F.flow_resampler_grouped(srcs[key], flow, group, self.grid_order)
+        out = self.decode(self.encode(image0, dimage0, group), disp, warp)
         self.gen_image1, self.flow_image1 = out.get("gen_image1"), out.get("flow_image1")
         self.gen_dimage1, self.flow_dimage1 = out.get("gen_dimage1"), out.get("flow_dimage1")
 
-    def encode(self, image0, dimage0):
-        """The per-modality pre-encoders, e2_0 .. e4_0 and fc1 -> features [B, 4096] bf16."""
+    def encode(self, image0, dimage0, group=1):
+        """The per-modality pre-encoders, e2_0 .. e4_0 and fc1 -> features [B * group, 4096] bf16 (each source's row repeated
+        ``group`` times)."""
         g = self.algo
         x = image0 if image0 is not None else dimage0
         B, H = x.shape[0], x.shape[1]
@@ -113,7 +123,7 @@ class Base_Prediction_Model(ModelBase):
         e3_0 = conv2d_msra(e3, 128, 3, 3, 1, 1, "e3_0", act=a, algo=g)
         e4 = conv2d_msra(e3_0, 256, 3, 3, 2, 2, "e4", act=a, algo=g)
         e4_0 = conv2d_msra(e4, 256, 3, 3, 1, 1, "e4_0", act=a, algo=g)
-        return linear_msra(F.reshape(e4_0, (B, h5 * h5 * 256)), 4096, "fc1", act=a, algo=g)
+        return linear_msra(F.reshape(e4_0, (B, h5 * h5 * 256)), 4096, "fc1", act=a, algo=g, group=group)
 
     def decode(self, e5, disp, warp=None):
         """features [N, 4096] (encode), disp [N, viewpoint_dim] bf16 -> {gen_image1, gen_dimage1} [N, H, H, C] and, with
@@ -144,12 +154,22 @@ class Base_Prediction_Model(ModelBase):
         return {k: v for k, v in out.items() if v is not None}
 
     def forward(self, image0, dimage0, disp):
-        """image0 [B,H,H,3], dimage0 [B,H,H,1] fp32 in [0,1], disp [B,V] -> dict(gen_image1, gen_dimage1)."""
+        """image0 [B,H,H,3], dimage0 [B,H,H,1] fp32 in [0,1], disp [B,V] -> dict(gen_image1, gen_dimage1).
+        disp [B,T,V]: T targets per source, outputs [B,T,H,H,C]."""
         self.gen_image1 = self.gen_dimage1 = self.loss = None
         self.store.new_anchor()
         self.image0, self.dimage0, self.disp = image0, dimage0, disp
-        with use_store(self.store):
-            self.buildModel(image0, dimage0, F.to_bf16(disp))
+        if disp.dim() == 3:
+            B, T = int(disp.shape[0]), int(disp.shape[1])
+            with use_store(self.store):
+                self.buildModel(image0, dimage0, F.to_bf16(disp.reshape(B * T, disp.shape[2])), T)
+            for k in ("gen_image1", "flow_image1", "gen_dimage1", "flow_dimage1"):
+                v = getattr(self, k)
+                if v is not None:
+                    setattr(self, k, v.reshape((B, T) + tuple(v.shape[1:])))
+        else:
+            with use_store(self.store):
+                self.buildModel(image0, dimage0, F.to_bf16(disp))
         out = {}
         if self.use_color:
             out["gen_image1"] = self.gen_image1
@@ -159,7 +179,7 @@ class Base_Prediction_Model(ModelBase):
 
     def build_loss(self, image1, dimage1):
         """main_model.py:144-154: loss = L(colour) + L(depth) * depth_lr_factor; mean over the global batch."""
-        n = image1.shape[0] * image1.shape[1] * image1.shape[2] * self.world_size
+        n = image1.numel() // image1.shape[-1] * self.world_size       # every target pixel: B*H*W (B*T*H*W with T targets)
         loss = None
         if self.use_color:
             loss = F.reconstruction_loss(self.gen_image1, image1, self.loss_mode, inv_count=1.0 / n, unit_upstream=True)
@@ -172,8 +192,9 @@ class Base_Prediction_Model(ModelBase):
 
     def input_spec(self):
         B, H = self.batch_size, self.image_shape[0]
-        return {"image0": (B, H, H, 3), "depth0": (B, H, H, 1), "image1": (B, H, H, 3), "depth1": (B, H, H, 1),
-                "disp": (B, self.viewpoint_dim)}
+        T = () if self.num_targets == 1 else (self.num_targets,)
+        return {"image0": (B, H, H, 3), "depth0": (B, H, H, 1), "image1": (B,) + T + (H, H, 3), "depth1": (B,) + T + (H, H, 1),
+                "disp": (B,) + T + (self.viewpoint_dim,)}
 
     def step_loss(self, batch):
         self.forward(batch["image0"], batch["depth0"], batch["disp"])

@@ -53,6 +53,10 @@ class MultiObjectAppFlow(ModelBase):
     INPUT_KEYS = tuple(BATCH_KEYS)
 
     def __init__(self, conf, load_tfrec=True, build_loss=True, device=None):
+        if int(conf.get("num_targets", 1)) > 1:
+            raise ValueError(
+                "%s trains one target per sample (num_targets = %s): its targets are per-object renders, masks and depths of "
+                "a multi-object scene, not viewpoints of one source image" % (type(self).__name__, conf["num_targets"]))
         self.conf = conf
         self.batch_size = int(conf["batch_size"])
         H = int(conf.get("image_size", 128))

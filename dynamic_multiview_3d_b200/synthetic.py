@@ -5,12 +5,15 @@ float32 NHWC images in [0,1] on the reference renderer's 0.5-grey background
 N(0, 0.02) noise; image1 is the same blob rotated by the sampled azimuth difference.
 Depth: 1.0 far plane, blob at 0.3-0.6.  Viewpoint: one-hot azimuth (V=19 bins of 20 deg) or
 the reference-native (d_elevation, d_azimuth) radians (collect_data_node.py:125-131).
+targets=T > 1: T target views per source at distinct azimuth bins, image1 [B, T, H, W, 3], disp [B, T, V] (depth1 /
+mask1 likewise).  Target 0 and everything else are the targets=1 batch of the same seed; the other targets are drawn
+after it.
 Host-side NumPy: this is input generation, not part of the measured path.
 """
 import numpy as np
 
 
-def make_batch(batch, size=224, viewpoint="onehot19", seed=1234, rank=0, depth=False, views=1):
+def make_batch(batch, size=224, viewpoint="onehot19", seed=1234, rank=0, depth=False, views=1, targets=1):
     rng = np.random.default_rng(seed + rank)
     H = W = size
     yy, xx = np.mgrid[0:H, 0:W].astype(np.float32)
@@ -33,6 +36,7 @@ def make_batch(batch, size=224, viewpoint="onehot19", seed=1234, rank=0, depth=F
     mask1 = np.zeros((batch, H, W, 1), np.float32)
     bins = rng.integers(0, 19, size=batch)
     disp = np.zeros((batch, 19 if viewpoint == "onehot19" else 2), np.float32)
+    scenes = []
     for b in range(batch):
         colour = rng.uniform(0.1, 0.9, size=3).astype(np.float32)
         jit = rng.uniform(-4, 4, size=2)
@@ -43,6 +47,7 @@ def make_batch(batch, size=224, viewpoint="onehot19", seed=1234, rank=0, depth=F
         dval = rng.uniform(0.3, 0.6)
         depth1[b, m1, 0] = dval
         mask1[b, m1, 0] = 1.0
+        scenes.append((yaw1 - daz, colour, jit, dval))
         for v in range(n_src):
             yaw0 = yaw1 - daz - np.deg2rad(10.0 * v)
             img0, m0 = blob(yaw0, colour, jit)
@@ -57,10 +62,39 @@ def make_batch(batch, size=224, viewpoint="onehot19", seed=1234, rank=0, depth=F
     image1 += rng.normal(0, 0.02, image1.shape).astype(np.float32)
     np.clip(image0, 0, 1, out=image0)
     np.clip(image1, 0, 1, out=image1)
+    if targets > 1:
+        image1, depth1, mask1, disp = _more_targets(rng, blob, scenes, bins, int(targets), viewpoint, image1, depth1, mask1, disp)
     out = {"image0": image0[:, 0] if views <= 1 else image0, "image1": image1, "disp": disp}
     if depth:
         out.update(depth0=depth0, depth1=depth1, mask1=mask1)
     return out
+
+
+def _more_targets(rng, blob, scenes, bins, T, viewpoint, image1, depth1, mask1, disp):
+    """Targets 1 .. T-1 of every source, at azimuth bins (relative to the source) other than target 0's and each other's."""
+    if T > 19:
+        raise ValueError("at most 19 targets per source (one per azimuth bin)")
+    B = len(scenes)
+    im = np.empty((B, T) + image1.shape[1:], np.float32)
+    dp = np.ones((B, T) + depth1.shape[1:], np.float32)
+    mk = np.zeros((B, T) + mask1.shape[1:], np.float32)
+    ds = np.zeros((B, T, disp.shape[1]), np.float32)
+    im[:, 0], dp[:, 0], mk[:, 0], ds[:, 0] = image1, depth1, mask1, disp
+    for b, (yaw0, colour, jit, dval) in enumerate(scenes):
+        others = rng.permutation(np.delete(np.arange(19), bins[b]))[:T - 1]
+        for t, k in enumerate(others, 1):
+            daz = np.deg2rad(20.0 * k)
+            img, m = blob(yaw0 + daz, colour, jit)
+            im[b, t] = img
+            dp[b, t, m, 0] = dval
+            mk[b, t, m, 0] = 1.0
+            if viewpoint == "onehot19":
+                ds[b, t, k] = 1.0
+            else:
+                ds[b, t] = (0.0, daz)
+    im[:, 1:] += rng.normal(0, 0.02, im[:, 1:].shape).astype(np.float32)
+    np.clip(im, 0, 1, out=im)
+    return im, dp, mk, ds
 
 
 def make_multiobject_batch(batch, size=128, seed=1234, rank=0):

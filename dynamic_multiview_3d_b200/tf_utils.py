@@ -79,14 +79,15 @@ def flow_resample_layer(src_img, flow_field, grid_order="ref_yx", name="tgt_img"
     return F.flow_resampler(src_img, flow_field, grid_order)
 
 
-def linear_msra(input_, output_size, name, act=None, algo=None):
-    """tf_utils.py:54-67: x @ Matrix[K,N] + b, Matrix ~ N(0, sqrt(2/K)), b = 0."""
+def linear_msra(input_, output_size, name, act=None, algo=None, group=1):
+    """tf_utils.py:54-67: x @ Matrix[K,N] + b, Matrix ~ N(0, sqrt(2/K)), b = 0.  group > 1: each output row is repeated
+    ``group`` times (functional.linear)."""
     store = current_store()
     fan_in = int(input_.shape[-1])
     with store.scope(name):
         matrix = store.get("Matrix", [fan_in, output_size], "normal", math.sqrt(2.0 / float(fan_in)))
         b = store.get("b", [output_size], "zeros")
-    return _rec(store, matrix, F.linear(input_, matrix, b, act, algo))
+    return _rec(store, matrix, F.linear(input_, matrix, b, act, algo, group))
 
 
 def conv2d_msra(input_, output_dim, k_h, k_w, d_h, d_w, name, act=None, algo=None, out_dtype=torch.bfloat16):

@@ -320,7 +320,7 @@ def synthetic_batch(model, seed, rank=0):
     elif isinstance(model, MultiObjectAppFlow):
         b = S.make_multiobject_batch(B, H, seed=seed, rank=rank)
     else:
-        b = S.make_batch(B, H, vp, seed=seed, rank=rank, depth=True)
+        b = S.make_batch(B, H, vp, seed=seed, rank=rank, depth=True, targets=getattr(model, "num_targets", 1))
     return {k: b[k] for k in model.INPUT_KEYS}
 
 
@@ -369,6 +369,10 @@ def main(argv=None):
     conf = load_conf(args.hyper)
     if args.num_iterations is not None:
         conf["num_iterations"] = args.num_iterations
+    if args.tfrecords and int(conf.get("num_targets", 1)) > 1:
+        raise SystemExit("--tfrecords trains one target per source: each record holds one (source, target) pair and names no "
+                         "object, so records cannot be grouped into several targets of one source; set num_targets = 1 or "
+                         "train on synthetic batches")
     if world > 1:
         import torch.distributed as dist
         torch.cuda.set_device(local)

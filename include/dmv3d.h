@@ -103,6 +103,21 @@ int dmv_sampler_fwd(const float* data, const float* wf, float* out, int32_t* dbg
 int dmv_sampler_fwd_shared_src(const float* data, int B_src, int group, const float* wf, float* out,
                                int H, int W, int C, int Hout, int Wout, unsigned flags, void* stream);
 
+/* ---- several targets of one source (multi-target training) ---- *
+ * Output sample n (0 <= n < B_src*group) warps data[n / group]: data [B_src,H,W,C] f32, wf / grad_wf [B_src*group,Hout,Wout,2],
+ * gen_out / target / grad_out [B_src*group,Hout,Wout,C].  No gradient wrt the source (it is a network input).  Every value
+ * has the bits of the plain call on the source repeated `group` times along the batch.  Refusals: DMV_E_INVALID_ARG for a
+ * null pointer or non-positive B_src / group, DMV_E_UNSUPPORTED_SHAPE when B_src*group overflows and as the plain call,
+ * DMV_E_ALIGN as the plain call; a refused call launches nothing.
+ *   dmv_sampler_loss_fused_shared_src: dmv_sampler_loss_fused; workspace dmv_sampler_loss_workspace_size(B_src*group, Hout, Wout).
+ *   dmv_sampler_grad_flow_shared_src:  the grad_wf half of dmv_sampler_bwd (grad_out = d loss / d out).                        */
+int dmv_sampler_loss_fused_shared_src(const float* data, int B_src, int group, const float* wf, const float* target,
+                                      const float* chan_weight, int mode, float inv_count, float* gen_out, float* grad_wf,
+                                      float* loss_out, int H, int W, int C, int Hout, int Wout, unsigned flags,
+                                      void* workspace, size_t workspace_bytes, void* stream);
+int dmv_sampler_grad_flow_shared_src(const float* data, int B_src, int group, const float* wf, const float* grad_out,
+                                     float* grad_wf, int H, int W, int C, int Hout, int Wout, unsigned flags, void* stream);
+
 /* replaces the registered gradient "ResamplerGrad" (implicit via
  * tf.train.AdamOptimizer.minimize, appearance_flow_model.py:77).
  *   grad_data [B,H,W,C] f32 or NULL (skip: the source is a network input)
@@ -232,6 +247,13 @@ int dmv_act_bwd(const void* dy, const void* y, void* dpre, int dtype, long long 
 size_t dmv_act_bwd_bias_workspace_size(long long rows, int C);
 int dmv_act_bwd_bias(const void* dy_bf16, const void* y_bf16, void* dpre_bf16, float* db, long long rows,
                      int C, int act, void* workspace, size_t workspace_bytes, void* stream);
+/* dmv_act_bwd_bias of a layer whose output [rows][C] was consumed `group` times (dy has rows * group rows, row r*group+t
+ * for use t; row pitch ld_dy >= C elements, ld_dy % 8 == 0, so dy may be a column slice of a wider gradient):
+ *   dpre[r][c] = bf16_rn((sum_{t = 0 .. group-1, in order, fp32} dy[r*group+t][c]) * act'(y[r][c])),  db = column sums of dpre.
+ * workspace: dmv_act_bwd_bias_workspace_size(rows, C).  At group = 1, ld_dy = C the bits of dmv_act_bwd_bias. */
+int dmv_act_bwd_bias_grouped(const void* dy_bf16, long long ld_dy, int group, const void* y_bf16, void* dpre_bf16,
+                             float* db, long long rows, int C, int act, void* workspace, size_t workspace_bytes,
+                             void* stream);
 /* Thin stride-2 layers (image side of e0, appearance_flow_model.py:88; 2-channel side of the flow head, :125) run on
  * X2[n][H/2][W/2][32] = the 2x2 pixel block as channels (ph, pw, c), zero padded, bf16.  The conv / deconv entry
  * points build X2 themselves from a DMV_DT_F32 / DMV_DT_BF16 tensor; a caller that keeps X2 between the forward
