@@ -35,6 +35,8 @@ SIGNATURES = {
     "dmv_sampler_loss_fused": (_i, [_vp, _vp, _vp, C.POINTER(_f), _i, _f, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _u, _vp, _sz, _vp]),
     "dmv_sampler_loss_fused_shared_src": (_i, [_vp, _i, _i, _vp, _vp, C.POINTER(_f), _i, _f, _vp, _vp, _vp, _i, _i, _i, _i, _i, _u, _vp, _sz, _vp]),
     "dmv_sampler_grad_flow_shared_src": (_i, [_vp, _i, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _u, _vp]),
+    "dmv_sampler_fuse_views_loss": (_i, [_vp, _i, _vp, _vp, C.POINTER(_f), _i, _f, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _u, _vp, _sz,
+                                         _vp]),
     "dmv_loss_workspace_size": (_sz, [_ll]),
     "dmv_loss_fused_fwd_bwd": (_i, [_vp, _vp, _i, _vp, _vp, C.POINTER(_f), _i, _f, _vp, _vp, _vp, _vp, _ll, _i, _vp, _sz, _vp]),
     "dmv_scale_by_device_scalar": (_i, [_vp, _vp, _ll, _vp]),

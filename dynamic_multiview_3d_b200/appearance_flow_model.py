@@ -15,12 +15,19 @@ reproduces the reference shapes and 224 gives BASELINE's.
 
 Extra conf keys (all optional): image_size (128), viewpoint_dim (2), loss ('l2' = reference,
 'l1' = north-star), grid_order ('ref_yx' = the reference's transposing (Y,X) grid, 'xy'),
-algo ('auto'|'simt'|'tcgen05'), seed (0), num_targets (1).
+algo ('auto'|'simt'|'tcgen05'), seed (0), num_targets (1), num_views (1).
 
 Several targets per source: a batch with disp [B, T, viewpoint_dim] and image1 [B, T, H, H, 3] trains B sources x T
 targets.  The encoder runs once per source, fc1 / e_fc1 hands each source's features to its T targets
 (functional.linear(group=T)), the decoder runs at B*T rows and the warp reads each source in place.  The loss is the
 mean over all B*T target images.  conf['num_targets'] only shapes input_spec(); batch_size is the number of sources.
+
+Several source views per target (conf['num_views'] = Vw > 1, Zhou et al.'s multi-view appearance flow, the batch layout
+of MultiViewFusionAppFlow): image0 [Vw, B, H, H, 3], disp [Vw, B, viewpoint_dim] (source v's viewpoint change to the
+target), image1 [B, H, H, 3].  Every view runs the same network (encoder and decoder at Vw*B rows); the flow head has a
+third channel, a per-pixel confidence logit, and the prediction is  sum_v softmax_v(logit) * warp(src_v, flow_v).  The
+warps, the fusion, the loss and the head gradient are one kernel (functional.fused_views_warp_loss).  gen is the fused
+[B, H, H, 3]; flow_field [Vw, B, H, H, 2] and confidence [Vw, B, H, H] are views of the head.
 """
 import os
 
@@ -31,6 +38,8 @@ from .model_base import ModelBase
 from .optimizer import TFAdam
 from .tf_utils import conv2d_msra, coords, deconv2d_msra, flow_resample_layer, linear_msra, warp_pts_layer
 from .variables import VariableStore, use_store
+
+MAX_VIEWS = 8          # dmv_sampler_fuse_views_loss fuses up to 8 source views
 
 
 class AppearanceFlowModel(ModelBase):
@@ -48,6 +57,15 @@ class AppearanceFlowModel(ModelBase):
         self.num_targets = int(conf.get("num_targets", 1))
         if self.num_targets < 1:
             raise ValueError("num_targets must be >= 1")
+        self.num_views = int(conf.get("num_views", 1))
+        if not 1 <= self.num_views <= MAX_VIEWS:
+            raise ValueError("%s: num_views must be 1 .. %d (the fused multi-view kernel's limit), got %d"
+                             % (type(self).__name__, MAX_VIEWS, self.num_views))
+        if self.num_views > 1 and self.num_targets > 1:
+            raise ValueError("%s trains several source views of one target (num_views = %d) or several targets of one source "
+                             "(num_targets = %d), not both" % (type(self).__name__, self.num_views, self.num_targets))
+        self.head_channels = 3 if self.num_views > 1 else 2      # flow, plus the confidence logit with several views
+        self.confidence = None
         self.loss_mode = conf.get("loss", "l2")
         self.grid_order = conf.get("grid_order", "ref_yx")
         self.algo = conf.get("algo", None)
@@ -74,12 +92,15 @@ class AppearanceFlowModel(ModelBase):
             self.optimizer = TFAdam(self.store, conf["learning_rate"])
 
     def _zeros_for_build(self):
-        B = self.batch_size
-        return (torch.zeros([B] + self.image_shape, dtype=torch.float32, device=self.device),
-                torch.zeros([B, self.viewpoint_dim], dtype=torch.float32, device=self.device))
+        lead = [self.batch_size] if self.num_views == 1 else [self.num_views, self.batch_size]
+        return (torch.zeros(lead + self.image_shape, dtype=torch.float32, device=self.device),
+                torch.zeros(lead + [self.viewpoint_dim], dtype=torch.float32, device=self.device))
 
     def input_spec(self):
         B = self.batch_size
+        if self.num_views > 1:
+            Vw = self.num_views
+            return {"image0": (Vw, B) + tuple(self.image_shape), "image1": (B,) + tuple(self.image_shape), "disp": (Vw, B, self.viewpoint_dim)}
         T = () if self.num_targets == 1 else (self.num_targets,)
         return {"image0": tuple([B] + self.image_shape), "image1": tuple([B] + list(T) + self.image_shape),
                 "disp": (B,) + T + (self.viewpoint_dim,)}
@@ -155,7 +176,7 @@ class AppearanceFlowModel(ModelBase):
         d1_0 = conv2d_msra(d1, 32, 5, 5, 1, 1, "d1_0", act=a, algo=g)
         self._last_decoder = d1_0            # subclasses hang further heads here (multi-view confidence)
         # flow head: no activation (appearance_flow_model.py:125); fp32 out for the sampler
-        return deconv2d_msra(d1_0, [B, H, H, 2], 5, 5, 2, 2, "flow_field", act=None, algo=g, out_dtype=torch.float32)
+        return deconv2d_msra(d1_0, [B, H, H, self.head_channels], 5, 5, 2, 2, "flow_field", act=None, algo=g, out_dtype=torch.float32)
 
     def forward(self, image0, disp, keep=None):
         """image0 [B,H,H,3] fp32 in [0,1], disp [B,V] fp32 -> dict(flow_field, gen); sets the
@@ -165,6 +186,11 @@ class AppearanceFlowModel(ModelBase):
         self.flow_field = self.gen = self.loss = None
         self.store.new_anchor()
         self.image0, self.disp = image0, disp
+        if self.num_views > 1:
+            with use_store(self.store):
+                head = self._views_head(image0, disp)
+            self._set_views(head, F.fused_views_warp(_flat_views(image0), head, self.num_views, self.grid_order))
+            return {"flow_field": self.flow_field, "gen": self.gen}
         if disp.dim() == 3:
             with use_store(self.store):
                 flow, T = self._grouped_flow(image0, disp)
@@ -182,6 +208,21 @@ class AppearanceFlowModel(ModelBase):
         if image0.shape[0] != B:
             raise ValueError("image0 holds %d sources, disp %d" % (image0.shape[0], B))
         return self.buildModel(image0, F.to_bf16(disp.reshape(B * T, disp.shape[2])), T), T
+
+    def _views_head(self, image0, disp):
+        """image0 [Vw,B,H,H,3], disp [Vw,B,V] -> the 3-channel head [Vw*B,H,H,3]: every view through the network."""
+        Vw, B = self.num_views, int(image0.shape[1]) if image0.dim() == 5 else -1
+        if image0.dim() != 5 or disp.dim() != 3 or tuple(image0.shape[:2]) != (Vw, B) or tuple(disp.shape[:2]) != (Vw, B):
+            raise ValueError("%s with num_views = %d takes image0 [%d, B, H, H, 3] and disp [%d, B, V], got %s and %s"
+                             % (type(self).__name__, Vw, Vw, Vw, tuple(image0.shape), tuple(disp.shape)))
+        return self.buildModel(_flat_views(image0), F.to_bf16(disp.reshape(Vw * B, disp.shape[2])))
+
+    def _set_views(self, head, fused):
+        Vw = self.num_views
+        lead = (Vw, head.shape[0] // Vw) + tuple(head.shape[1:3])
+        self.flow_field = head[..., :2].reshape(lead + (2,))
+        self.confidence = head[..., 2].reshape(lead)
+        self.gen = fused
 
     @property
     def warp_pts(self):
@@ -207,6 +248,8 @@ class AppearanceFlowModel(ModelBase):
                 or self.device.type == "meta":
             self.forward(image0, disp)
             return self.build_loss(image1)
+        if self.num_views > 1:
+            return self._views_forward_and_loss(image0, image1, disp)
         if disp.dim() == 3:
             return self._grouped_forward_and_loss(image0, image1, disp)
         self.flow_field = self.gen = self.loss = None
@@ -242,10 +285,28 @@ class AppearanceFlowModel(ModelBase):
         self.flow_field, self.gen = _per_source(flow, T), _per_source(gen, T)
         return self.loss
 
+    def _views_forward_and_loss(self, image0, image1, disp):
+        """forward_and_loss with Vw source views per target: every view's warp, the confidence fusion, the loss and the
+        gradient wrt the 3-channel head in one kernel (dmv_sampler_fuse_views_loss); under no_grad the loss alone."""
+        self.flow_field = self.gen = self.loss = self.confidence = None
+        self.store.new_anchor()
+        self.image0, self.disp, self.image1 = image0, disp, image1
+        with use_store(self.store):
+            head = self._views_head(image0, disp)
+        n = image1.shape[0] * image1.shape[1] * image1.shape[2] * self.world_size
+        self.loss, fused = F.fused_views_warp_loss(_flat_views(image0), head, image1, self.num_views, self.loss_mode, inv_count=1.0 / n,
+                                                   grid_order=self.grid_order, unit_upstream=True)
+        self._set_views(head, fused)
+        return self.loss
+
     def step_loss(self, batch):
         return self.forward_and_loss(batch["image0"], batch["image1"], batch["disp"])
 
     def render_sources(self):
+        if self.num_views > 1:
+            raise NotImplementedError(
+                "%s with num_views = %d has no render(): each view it predicts fuses the warps of %d source views by predicted "
+                "confidences, and rendering decodes one source per sample" % (type(self).__name__, self.num_views, self.num_views))
         return ("image0",)
 
     def _render_encode(self, sources):
@@ -259,9 +320,16 @@ class AppearanceFlowModel(ModelBase):
         """appearance_flow_model.py:132-179: output / ground-truth / input grids, the flow image and the
         correspondence probes (visualize.py).  The TF session argument becomes the batch itself."""
         from .visualize import visualize
+        if self.num_views > 1:               # several source views: source frame 0, the fused prediction, the target
+            return visualize(self, image0, image1, disp, iter_num, source=image0[0])
         if disp.dim() == 3:                  # several targets per source: each source's first
             image1, disp = image1[:, 0], disp[:, 0]
         return visualize(self, image0, image1, disp, iter_num)
+
+
+def _flat_views(x):
+    """[Vw, B, ...] -> [Vw*B, ...] (view-major rows, no copy)"""
+    return x.reshape((x.shape[0] * x.shape[1],) + tuple(x.shape[2:]))
 
 
 def _per_source(x, T):
@@ -322,4 +390,4 @@ class AppearanceFlowTinghui(AppearanceFlowModel):
         d = deconv2d_msra(d, [B, H // 4, H // 4, 64], 3, 3, 2, 2, "d2", act="relu", algo=g)
         d = deconv2d_msra(d, [B, H // 2, H // 2, 32], 3, 3, 2, 2, "d1", act="relu", algo=g)
         d = deconv2d_msra(d, [B, H, H, 16], 3, 3, 2, 2, "d0", act="relu", algo=g)
-        return deconv2d_msra(d, [B, H, H, 2], 3, 3, 1, 1, "flow_field", act=None, algo=g, out_dtype=torch.float32)
+        return deconv2d_msra(d, [B, H, H, self.head_channels], 3, 3, 1, 1, "flow_field", act=None, algo=g, out_dtype=torch.float32)

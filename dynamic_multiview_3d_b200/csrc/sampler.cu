@@ -1027,6 +1027,326 @@ int sampler_loss_fused(const float* data, int B_src, int group, const float* wf,
     return check_launch("sampler_loss_fused");
 }
 
+// ---------------------------------------------------------------------------------------------
+// Several source views per target (dmv_sampler_fuse_views_loss): one CTA per 32x32 TARGET tile.  The head of view v is
+// [Hout, Wout, 3] (flow in channels 0-1, confidence logit in channel 2) and is read in place.  Arithmetic is that of the
+// composition it replaces -- sampler_tma_kernel MODE 0 per view, loss_kernel (loss.cu) with V = views, MODE 1 on its
+// grad_gen -- op for op, including the FMAs nvcc forms in loss_kernel under -fmad=true (the fusion sum and the logit
+// gradient), so fused_out and grad_head have the composition's bits.
+//   pass 0: softmax statistics (max, sum of __expf in view order, one reciprocal) per pixel, kept in registers;
+//   pass 1: per view, reduce the tap box, stage that view's window (36^2 / 44^2 box, or global gathers), accumulate the
+//           fused tile in shared memory; then the loss and dL/dfused (stored over the target tile);
+//   pass 2: per view, in reverse order, restage the window (L2-resident: the first pass just read it) and form the flow
+//           and logit gradients.  Keeping every view's window resident instead would take up to 8 x 31 KB of shared
+//           memory (C = 4), one CTA per SM; the reverse order reuses the last window of pass 1, so one view stages once.
+constexpr int kMaxViews = 8;
+
+struct ViewsArgs {
+    const float* head;
+    float* grad_head;
+    float w[4];
+    float inv_count;
+    int mode, views;
+    bool store_fused;
+    double* partials;
+    unsigned* counter;
+    float* loss_out;
+};
+
+// sample of head pixel hp (flow in channels 0-1), grid added as in sampler_tma_kernel
+__device__ __forceinline__ void head_sample(const float* __restrict__ head, long long hp, bool inb, int i, int j, const Geom& g,
+                                            float& sx, float& sy, bool& valid, int& fx, int& fy) {
+    float f0 = 0.f, f1 = 0.f;
+    if (inb) { f0 = __ldg(head + hp * 3); f1 = __ldg(head + hp * 3 + 1); }
+    sx = f0; sy = f1;
+    if (g.flags & DMV_SAMPLER_ADD_GRID) {
+        if (g.flags & DMV_SAMPLER_GRID_XY) {
+            sx = __fadd_rn(f0, (float)j);
+            sy = __fadd_rn(f1, (float)i);
+        } else {
+            sx = __fadd_rn(f0, (float)i);
+            sy = __fadd_rn(f1, (float)j);
+        }
+    }
+    valid = inb && (sx > -1.0f) && (sy > -1.0f) && (sx < (float)g.W) && (sy < (float)g.H);
+    fx = valid ? __float2int_rd(sx) : 0;
+    fy = valid ? __float2int_rd(sy) : 0;
+}
+
+// the staged window of one view: the smallest box that holds its tap box, or none (global gathers)
+struct Window {
+    bool staged;
+    int xa, ylo, pitch;
+};
+
+__device__ __forceinline__ Window view_window(const int* box, int C) {
+    Window w;
+    const int xlo = box[0], xhi = box[1], ylo = box[2], yhi = box[3];
+    w.xa = (C == 4) ? xlo : (xlo & ~3);
+    w.ylo = ylo;
+    const int span = max(xhi - w.xa, yhi - ylo);
+    w.staged = (xlo <= xhi) && (span < kBoxL);
+    w.pitch = ((span < kBoxS) ? kBoxS : kBoxL) * C;
+    return w;
+}
+
+template <int C>
+__device__ __forceinline__ void stage_window(const Window& w, float* s_win, const CUtensorMap* map_s, const CUtensorMap* map_l,
+                                             uint64_t* bar, unsigned& phase, int img) {
+    if (!w.staged) return;
+    if (threadIdx.x == 0) {
+        const int box = w.pitch / C;
+        tc::mbar_expect_tx(bar, box * box * C * 4);
+        tc::tma_load_3d(s_win, box == kBoxS ? map_s : map_l, bar, w.xa * C, w.ylo, img);
+    }
+    tc::mbar_wait(bar, phase);
+    phase ^= 1u;
+}
+
+// the four taps of a sample (sampler_tma_kernel's two window paths) and the bilinear value (MODE 0's op order)
+template <int C>
+__device__ __forceinline__ void view_taps(const Window& w, const float* s_win, const float* __restrict__ data, int img, const Geom& g,
+                                          bool valid, int fx, int fy, float (&p_ff)[C], float (&p_cf)[C], float (&p_fc)[C],
+                                          float (&p_cc)[C]) {
+    if (w.staged) {
+        const float* t = s_win + (valid ? (fy - w.ylo) * w.pitch + (fx - w.xa) * C : 0);
+#pragma unroll
+        for (int c = 0; c < C; ++c) {
+            p_ff[c] = t[c]; p_cf[c] = t[C + c]; p_fc[c] = t[w.pitch + c]; p_cc[c] = t[w.pitch + C + c];
+        }
+    } else {
+        const int cx = fx + 1, cy = fy + 1;
+        const bool fxi = fx >= 0, cxi = cx <= g.W - 1, fyi = fy >= 0, cyi = cy <= g.H - 1;
+        const float* base = data + (((long long)img * g.H + fy) * g.W + fx) * C;
+        const int rowf = g.W * C;
+#pragma unroll
+        for (int c = 0; c < C; ++c) {
+            p_ff[c] = (valid && fxi && fyi) ? __ldg(base + c) : 0.f;
+            p_cf[c] = (valid && cxi && fyi) ? __ldg(base + C + c) : 0.f;
+            p_fc[c] = (valid && fxi && cyi) ? __ldg(base + rowf + c) : 0.f;
+            p_cc[c] = (valid && cxi && cyi) ? __ldg(base + rowf + C + c) : 0.f;
+        }
+    }
+}
+
+template <int C, bool TRAIN>
+__global__ void __launch_bounds__(kThreads, 3) sampler_views_kernel(
+    const __grid_constant__ CUtensorMap map_src, const __grid_constant__ CUtensorMap map_src_l,
+    const __grid_constant__ CUtensorMap map_fused, const __grid_constant__ CUtensorMap map_tgt, const float* __restrict__ data,
+    Geom g, const ViewsArgs va) {
+    extern __shared__ __align__(128) float s_dyn[];
+    float* s_win = s_dyn;                              // one view's source window
+    float* s_fused = s_dyn + win_floats(C);            // [32][32 * C] fused tile
+    float* s_tgt = s_fused + 32 * 32 * C;              // TRAIN: target tile, then dL/dfused
+    __shared__ __align__(8) uint64_t s_bar[2];
+    __shared__ int s_box[kMaxViews][4];
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int V = va.views;
+    int b, i0, j0;
+    tile_origin(g, blockIdx.x, b, i0, j0);
+    if (tid < kMaxViews * 4) s_box[tid >> 2][tid & 3] = (tid & 1) ? -0x7fffffff : 0x7fffffff;
+    if (tid == 0) {
+        tc::mbar_init(&s_bar[0], 1);
+        tc::mbar_init(&s_bar[1], 1);
+        tc::fence_barrier_init();
+        tc::fence_proxy_async();
+        if (TRAIN) {
+            tc::mbar_expect_tx(&s_bar[1], 32 * 32 * C * 4);
+            tc::tma_load_3d(s_tgt, &map_tgt, &s_bar[1], j0 * C, i0, b);
+        }
+    }
+    __syncthreads();
+    const int j = j0 + lane;
+    const long long plane = (long long)g.B * g.Ho * g.Wo;              // head pixels per view
+    const long long pix0 = (long long)b * g.Ho * g.Wo;
+    // pass 0: softmax statistics, loss_kernel's order
+    float mx[kPPT], inv[kPPT];
+#pragma unroll
+    for (int k = 0; k < kPPT; ++k) {
+        const int i = i0 + warp + k * kWarps;
+        mx[k] = -INFINITY;
+        inv[k] = 1.0f;
+        if (V == 1 || i >= g.Ho || j >= g.Wo) continue;
+        const float* lp = va.head + (pix0 + (long long)i * g.Wo + j) * 3 + 2;
+        for (int v = 0; v < V; ++v) mx[k] = fmaxf(mx[k], __ldg(lp + v * plane * 3));
+        float den = 0.f;
+        for (int v = 0; v < V; ++v) den = __fadd_rn(den, __expf(__fsub_rn(__ldg(lp + v * plane * 3), mx[k])));
+        inv[k] = 1.0f / den;
+    }
+
+    // pass 1: the fused tile
+    unsigned phase = 0;
+    for (int v = 0; v < V; ++v) {
+        const int img = v * g.B + b;
+        float sx[kPPT], sy[kPPT];
+        bool valid[kPPT];
+        int fx[kPPT], fy[kPPT];
+        int bxlo = 0x7fffffff, bxhi = -0x7fffffff, bylo = 0x7fffffff, byhi = -0x7fffffff;
+#pragma unroll
+        for (int k = 0; k < kPPT; ++k) {
+            const int i = i0 + warp + k * kWarps;
+            head_sample(va.head, (long long)img * g.Ho * g.Wo + (long long)i * g.Wo + j, (i < g.Ho) && (j < g.Wo), i, j, g, sx[k], sy[k],
+                        valid[k], fx[k], fy[k]);
+            if (valid[k]) {
+                bxlo = min(bxlo, fx[k]); bxhi = max(bxhi, fx[k] + 1);
+                bylo = min(bylo, fy[k]); byhi = max(byhi, fy[k] + 1);
+            }
+        }
+        bxlo = __reduce_min_sync(0xffffffffu, bxlo); bxhi = __reduce_max_sync(0xffffffffu, bxhi);
+        bylo = __reduce_min_sync(0xffffffffu, bylo); byhi = __reduce_max_sync(0xffffffffu, byhi);
+        if (lane == 0) {
+            atomicMin(&s_box[v][0], bxlo); atomicMax(&s_box[v][1], bxhi);
+            atomicMin(&s_box[v][2], bylo); atomicMax(&s_box[v][3], byhi);
+        }
+        __syncthreads();              // the box is complete and every thread is done with the previous view's window
+        const Window w = view_window(s_box[v], C);
+        stage_window<C>(w, s_win, &map_src, &map_src_l, &s_bar[0], phase, img);
+#pragma unroll
+        for (int k = 0; k < kPPT; ++k) {
+            const int r = warp + k * kWarps, i = i0 + r;
+            if (i >= g.Ho || j >= g.Wo) continue;
+            float p_ff[C], p_cf[C], p_fc[C], p_cc[C];
+            view_taps<C>(w, s_win, data, img, g, valid[k], fx[k], fy[k], p_ff, p_cf, p_fc, p_cc);
+            const float dx = valid[k] ? __fsub_rn((float)(fx[k] + 1), sx[k]) : 0.f;
+            const float dy = valid[k] ? __fsub_rn((float)(fy[k] + 1), sy[k]) : 0.f;
+            const float omdx = __fsub_rn(1.0f, dx), omdy = __fsub_rn(1.0f, dy);
+            const float w_ff = __fmul_rn(dx, dy), w_cc = __fmul_rn(omdx, omdy), w_fc = __fmul_rn(dx, omdy), w_cf = __fmul_rn(omdx, dy);
+            float sm = 1.0f;
+            if (V > 1)
+                sm = __fmul_rn(__expf(__fsub_rn(__ldg(va.head + ((long long)img * g.Ho * g.Wo + (long long)i * g.Wo + j) * 3 + 2), mx[k])), inv[k]);
+            float* fu = s_fused + (r * 32 + lane) * C;
+#pragma unroll
+            for (int c = 0; c < C; ++c) {
+                float gv = __fmul_rn(w_ff, p_ff[c]);
+                gv = __fadd_rn(gv, __fmul_rn(w_cc, p_cc[c]));
+                gv = __fadd_rn(gv, __fmul_rn(w_fc, p_fc[c]));
+                gv = __fadd_rn(gv, __fmul_rn(w_cf, p_cf[c]));
+                gv = valid[k] ? gv : 0.f;
+                fu[c] = (V == 1) ? gv : __fmaf_rn(sm, gv, v == 0 ? 0.f : fu[c]);
+            }
+        }
+    }
+    if (va.store_fused) {
+        tc::fence_proxy_async();          // generic-proxy writes of s_fused -> visible to the bulk store
+        __syncthreads();
+        if (tid == 0) tc::tma_store_3d(&map_fused, s_fused, j0 * C, i0, b);
+    }
+    if (TRAIN) {
+        // loss and dL/dfused per pixel as dmv_loss_fused_fwd_bwd (mask = 1); dL/dfused replaces the target in shared memory
+        tc::mbar_wait(&s_bar[1], 0);
+        double local = 0.0;
+#pragma unroll
+        for (int k = 0; k < kPPT; ++k) {
+            const int r = warp + k * kWarps;
+            if (i0 + r >= g.Ho || j >= g.Wo) continue;
+            const float* fu = s_fused + (r * 32 + lane) * C;
+            float* tg = s_tgt + (r * 32 + lane) * C;
+            float acc = 0.f;
+#pragma unroll
+            for (int c = 0; c < C; ++c) {
+                const float d = __fsub_rn(fu[c], tg[c]);
+                float gq;
+                if (va.mode == DMV_LOSS_L2) {
+                    acc = __fadd_rn(acc, __fmul_rn(__fmul_rn(va.w[c], d), d));
+                    gq = __fadd_rn(d, d);
+                } else {
+                    acc = __fadd_rn(acc, __fmul_rn(va.w[c], fabsf(d)));
+                    gq = (d > 0.f) ? 1.0f : (d < 0.f ? -1.0f : 0.0f);
+                }
+                // one view: loss_flat_kernel's (g * w) * inv_count; several: loss_kernel's g * (w * mask * inv_count)
+                tg[c] = (V == 1) ? __fmul_rn(__fmul_rn(gq, va.w[c]), va.inv_count) : __fmul_rn(gq, __fmul_rn(va.w[c], va.inv_count));
+            }
+            local += (double)acc;
+        }
+
+        // pass 2: flow and logit gradients, views in reverse order (the last window of pass 1 is still staged)
+        if (va.grad_head) {
+            for (int v = V - 1; v >= 0; --v) {
+                const int img = v * g.B + b;
+                const Window w = view_window(s_box[v], C);
+                if (v != V - 1) {
+                    __syncthreads();          // every thread is done with the previous view's window
+                    stage_window<C>(w, s_win, &map_src, &map_src_l, &s_bar[0], phase, img);
+                }
+#pragma unroll
+                for (int k = 0; k < kPPT; ++k) {
+                    const int r = warp + k * kWarps, i = i0 + r;
+                    if (i >= g.Ho || j >= g.Wo) continue;
+                    const long long hp = (long long)img * g.Ho * g.Wo + (long long)i * g.Wo + j;
+                    float sx, sy;
+                    bool valid;
+                    int fx, fy;
+                    head_sample(va.head, hp, true, i, j, g, sx, sy, valid, fx, fy);
+                    float p_ff[C], p_cf[C], p_fc[C], p_cc[C];
+                    view_taps<C>(w, s_win, data, img, g, valid, fx, fy, p_ff, p_cf, p_fc, p_cc);
+                    const float dx = valid ? __fsub_rn((float)(fx + 1), sx) : 0.f;
+                    const float dy = valid ? __fsub_rn((float)(fy + 1), sy) : 0.f;
+                    const float omdx = __fsub_rn(1.0f, dx), omdy = __fsub_rn(1.0f, dy);
+                    const float w_ff = __fmul_rn(dx, dy), w_cc = __fmul_rn(omdx, omdy), w_fc = __fmul_rn(dx, omdy), w_cf = __fmul_rn(omdx, dy);
+                    float sm = 1.0f;
+                    if (V > 1) sm = __fmul_rn(__expf(__fsub_rn(__ldg(va.head + hp * 3 + 2), mx[k])), inv[k]);
+                    const float* fu = s_fused + (r * 32 + lane) * C;
+                    const float* gf = s_tgt + (r * 32 + lane) * C;
+                    float g0 = 0.f, g1 = 0.f, gl = 0.f;
+#pragma unroll
+                    for (int c = 0; c < C; ++c) {
+                        // grad_gen = softmax * dL/dfused, and the logit term, as loss_kernel
+                        const float gc = (V == 1) ? gf[c] : __fmul_rn(sm, gf[c]);
+                        if (V > 1) {
+                            float gv = __fmul_rn(w_ff, p_ff[c]);
+                            gv = __fadd_rn(gv, __fmul_rn(w_cc, p_cc[c]));
+                            gv = __fadd_rn(gv, __fmul_rn(w_fc, p_fc[c]));
+                            gv = __fadd_rn(gv, __fmul_rn(w_cf, p_cf[c]));
+                            gv = valid ? gv : 0.f;
+                            gl = __fmaf_rn(gf[c], __fsub_rn(gv, fu[c]), gl);
+                        }
+                        // grad wrt the flow through that grad_gen, as MODE 1
+                        const float a0 = __fadd_rn(__fmul_rn(omdy, __fsub_rn(p_cc[c], p_fc[c])), __fmul_rn(dy, __fsub_rn(p_cf[c], p_ff[c])));
+                        const float a1 = __fadd_rn(__fmul_rn(omdx, __fsub_rn(p_cc[c], p_cf[c])), __fmul_rn(dx, __fsub_rn(p_fc[c], p_ff[c])));
+                        g0 = __fadd_rn(g0, __fmul_rn(gc, a0));
+                        g1 = __fadd_rn(g1, __fmul_rn(gc, a1));
+                    }
+                    float* gh = va.grad_head + hp * 3;
+                    gh[0] = valid ? g0 : 0.f;
+                    gh[1] = valid ? g1 : 0.f;
+                    gh[2] = (V > 1) ? __fmul_rn(sm, gl) : 0.f;     // one view: the softmax is constant
+                }
+            }
+        }
+
+        // deterministic loss, as MODE 2: fixed tree in the CTA, per-CTA partials, ordered sum by the last CTA
+        __shared__ double s_red[kWarps];
+        __shared__ bool s_last;
+        for (int o = 16; o > 0; o >>= 1) local += __shfl_down_sync(0xffffffffu, local, o);
+        if (lane == 0) s_red[warp] = local;
+        __syncthreads();
+        if (tid == 0) {
+            double t = 0.0;
+            for (int q = 0; q < kWarps; ++q) t += s_red[q];
+            va.partials[blockIdx.x] = t;
+            __threadfence();
+            s_last = (atomicAdd(va.counter, 1u) == gridDim.x - 1);
+        }
+        __syncthreads();
+        if (s_last) {
+            __threadfence();
+            double t = 0.0;
+            for (unsigned q = tid; q < gridDim.x; q += kThreads) t += __ldcg(va.partials + q);
+            for (int o = 16; o > 0; o >>= 1) t += __shfl_down_sync(0xffffffffu, t, o);
+            __syncthreads();
+            if (lane == 0) s_red[warp] = t;
+            __syncthreads();
+            if (tid == 0) {
+                double tot = 0.0;
+                for (int q = 0; q < kWarps; ++q) tot += s_red[q];
+                *va.loss_out = (float)(tot * (double)va.inv_count);
+                *va.counter = 0;
+            }
+        }
+    }
+    if (va.store_fused && tid == 0) tc::bulk_commit_wait_read();   // the tile stays in shared memory until the store has read it
+}
+
 }  // namespace
 
 extern "C" {
@@ -1044,6 +1364,71 @@ int dmv_sampler_loss_fused_shared_src(const float* data, int B_src, int group, c
                                       size_t workspace_bytes, void* stream) {
     return sampler_loss_fused(data, B_src, group, wf, target, chan_weight, mode, inv_count, gen_out, grad_wf, loss_out, H, W, C, Hout, Wout,
                               flags, workspace, workspace_bytes, stream);
+}
+
+int dmv_sampler_fuse_views_loss(const float* data, int views, const float* head, const float* target, const float* chan_weight, int mode,
+                                float inv_count, float* fused_out, float* grad_head, float* loss_out, int B, int H, int W, int C, int Hout,
+                                int Wout, unsigned flags, void* workspace, size_t workspace_bytes, void* stream) {
+    DMV_REQUIRE(data && head, DMV_E_INVALID_ARG, "sampler_fuse_views_loss: null pointer");
+    const bool train = target != nullptr;
+    if (train) {
+        DMV_REQUIRE(chan_weight && loss_out, DMV_E_INVALID_ARG, "sampler_fuse_views_loss: training needs chan_weight and loss_out");
+        DMV_REQUIRE(mode == DMV_LOSS_L2 || mode == DMV_LOSS_L1, DMV_E_INVALID_ARG, "sampler_fuse_views_loss: unknown loss mode");
+    } else {
+        DMV_REQUIRE(fused_out && !grad_head && !loss_out, DMV_E_INVALID_ARG,
+                    "sampler_fuse_views_loss: forward only (target NULL) writes fused_out alone: grad_head and loss_out must be NULL");
+    }
+    DMV_REQUIRE(views >= 1 && views <= kMaxViews, DMV_E_UNSUPPORTED_SHAPE, "sampler_fuse_views_loss: need 1 <= views <= 8");
+    DMV_REQUIRE(C == 1 || C == 3 || C == 4, DMV_E_UNSUPPORTED_SHAPE, "sampler_fuse_views_loss: need C in {1,3,4}");
+    DMV_REQUIRE((long long)views * B < (1ll << 31), DMV_E_UNSUPPORTED_SHAPE, "sampler_fuse_views_loss: views * B beyond int");
+    Geom g;
+    int rc = make_geom(g, B, H, W, C, Hout, Wout, flags);
+    if (rc) return rc;
+    DMV_REQUIRE(g.tw_shift == 5 && ((W * C) & 3) == 0 && ((Wout * C) & 3) == 0, DMV_E_UNSUPPORTED_SHAPE,
+                "sampler_fuse_views_loss: needs image-shaped output (Hout > 1) and W*C, Wout*C multiples of 4");
+    DMV_REQUIRE((((uintptr_t)data | (uintptr_t)head | (uintptr_t)target | (uintptr_t)fused_out | (uintptr_t)grad_head) & 15) == 0, DMV_E_ALIGN,
+                "sampler_fuse_views_loss: buffers must be 16-byte aligned");
+    const int grid = g.B * g.tiles_x * g.tiles_y;
+    if (train)
+        DMV_REQUIRE(workspace && workspace_bytes >= dmv_sampler_loss_workspace_size(B, Hout, Wout) && ((uintptr_t)workspace & 7) == 0,
+                    DMV_E_WORKSPACE, "sampler_fuse_views_loss: workspace too small or unaligned (it must be zeroed once and not shared)");
+    CUtensorMap map_src, map_src_l, map_fused, map_tgt;
+    rc = encode_f32_map(&map_src, data, W * C, H, views * B, kBoxS * C, kBoxS);
+    if (!rc) rc = encode_f32_map(&map_src_l, data, W * C, H, views * B, kBoxL * C, kBoxL);
+    if (!rc && fused_out) rc = encode_f32_map(&map_fused, fused_out, Wout * C, Hout, B, 32 * C, 32);
+    if (!rc && train) rc = encode_f32_map(&map_tgt, target, Wout * C, Hout, B, 32 * C, 32);
+    if (rc) return rc;
+    if (!fused_out) map_fused = map_src;              // not read: only a valid map to pass
+    if (!train) map_tgt = map_src;
+    ViewsArgs va;
+    va.head = head; va.grad_head = grad_head;
+    for (int c = 0; c < 4; ++c) va.w[c] = (train && c < C) ? chan_weight[c] : 0.f;
+    va.inv_count = inv_count; va.mode = mode; va.views = views; va.store_fused = fused_out != nullptr;
+    va.counter = train ? reinterpret_cast<unsigned*>(workspace) : nullptr;
+    va.partials = train ? reinterpret_cast<double*>(reinterpret_cast<char*>(workspace) + 16) : nullptr;
+    va.loss_out = loss_out;
+    const size_t wsm = (size_t)(win_floats(C) + (train ? 2 : 1) * 32 * 32 * C) * sizeof(float);
+    cudaStream_t st = (cudaStream_t)stream;
+#define DMV_LAUNCH_VIEWS(CT, TR)                                                                                   \
+    do {                                                                                                          \
+        static bool attr_done = false;                                                                            \
+        if (!attr_done) {                                                                                         \
+            cudaFuncSetAttribute(sampler_views_kernel<CT, TR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsm); \
+            attr_done = true;                                                                                     \
+        }                                                                                                         \
+        sampler_views_kernel<CT, TR><<<grid, kThreads, wsm, st>>>(map_src, map_src_l, map_fused, map_tgt, data, g, va); \
+    } while (0)
+    if (train) {
+        if (C == 1) DMV_LAUNCH_VIEWS(1, true);
+        else if (C == 3) DMV_LAUNCH_VIEWS(3, true);
+        else DMV_LAUNCH_VIEWS(4, true);
+    } else {
+        if (C == 1) DMV_LAUNCH_VIEWS(1, false);
+        else if (C == 3) DMV_LAUNCH_VIEWS(3, false);
+        else DMV_LAUNCH_VIEWS(4, false);
+    }
+#undef DMV_LAUNCH_VIEWS
+    return check_launch("sampler_loss_fused");
 }
 
 }  // extern "C"

@@ -1014,6 +1014,89 @@ def flow_resample_loss(data, flow, target, mode="l2", weights=None, inv_count=No
     return _WarpLoss.apply(data, flow, target, flags, tuple(weights), mode, inv_count, unit_upstream, group)
 
 
+class _ViewsWarpLoss(torch.autograd.Function):
+    """head -> (loss, fused): every view's warp by channels 0-1 of its head, the softmax fusion by channel 2, the loss
+    and d loss / d head in one kernel (dmv_sampler_fuse_views_loss).  The sources and the target are network inputs."""
+
+    @staticmethod
+    def forward(ctx, data, head, target, views, flags, weights, mode, inv_count, unit_upstream, want_grad):
+        Cc = data.shape[-1]
+        B, Ho, Wo = target.shape[0], target.shape[1], target.shape[2]
+        fused = torch.empty((B, Ho, Wo, Cc), dtype=torch.float32, device=data.device)
+        grad_head = torch.empty_like(head) if want_grad else None       # a validation pass computes the loss alone
+        loss = torch.empty((), dtype=torch.float32, device=data.device)
+        w = (C.c_float * Cc)(*[float(x) for x in weights])
+        nws = _lib.load().dmv_sampler_loss_workspace_size(B, Ho, Wo)
+        key = ("warp_loss", data.device.type, data.device.index)
+        ws = _loss_wss.get(key)
+        if ws is None or ws.numel() < nws:             # zeroed once: holds a self-resetting counter
+            ws = _loss_wss[key] = torch.zeros(int(nws), dtype=torch.uint8, device=data.device)
+        _tag[0] = "warp_loss"
+        call("dmv_sampler_fuse_views_loss", _p(data), views, _p(head), _p(target), w, LOSS[mode], float(inv_count), _p(fused),
+             _p(grad_head), _p(loss), B, data.shape[1], data.shape[2], Cc, Ho, Wo, flags, _p(ws), ws.numel(), _stream(data))
+        ctx.grad_head, ctx.unit_upstream = grad_head, unit_upstream
+        ctx.mark_non_differentiable(fused)
+        return loss, fused
+
+    @staticmethod
+    def backward(ctx, gloss, _gfused):
+        gh = ctx.grad_head
+        if not ctx.unit_upstream:
+            _tag[0] = "warp_loss"
+            call("dmv_scale_by_device_scalar", _p(gh), _p(gloss.contiguous().to(torch.float32)), gh.numel(), _stream(gh))
+        return None, gh, None, None, None, None, None, None, None, None
+
+
+def _views_args(data, head, views, grid_order, target=None):
+    if grid_order not in ("ref_yx", "xy"):
+        raise ValueError(grid_order)
+    _need_cuda(data, head, *([target] if target is not None else []))
+    views = int(views)
+    if data.dim() != 4 or head.dim() != 4 or head.shape[-1] != 3:
+        raise ValueError("data [views*B,H,W,C] and head [views*B,Hout,Wout,3] expected, got %s and %s"
+                         % (tuple(data.shape), tuple(head.shape)))
+    if views < 1 or head.shape[0] != data.shape[0] or data.shape[0] % views:
+        raise ValueError("data and head hold %d and %d rows, not views * B with views = %d" % (data.shape[0], head.shape[0], views))
+    if target is not None and (target.shape[0] * views != data.shape[0] or tuple(target.shape[1:3]) != tuple(head.shape[1:3])
+                               or target.shape[-1] != data.shape[-1]):
+        raise ValueError("target %s does not match data %s and head %s" % (tuple(target.shape), tuple(data.shape), tuple(head.shape)))
+    tensors = [data, head] + ([target] if target is not None else [])
+    if any(t.dtype != torch.float32 for t in tensors):
+        raise TypeError("the multi-view warp runs in float32 (reference precision)")
+    return views, SAMPLER_ADD_GRID | (SAMPLER_GRID_XY if grid_order == "xy" else 0)
+
+
+def fused_views_warp_loss(data, head, target, views, mode="l2", weights=None, inv_count=None, grid_order="ref_yx", unit_upstream=False):
+    """(loss, fused) of several source views per target (Zhou et al.'s multi-view appearance flow), view v of target b in
+    row v*B + b: data [views*B,H,W,C], head [views*B,Hout,Wout,3] (flow in channels 0-1, confidence logit in 2), target
+    [B,Hout,Wout,C].  fused = sum_v softmax_v(logit) * warp(data_v, flow_v); backward gives d loss / d head, all three
+    channels.  One launch (dmv_sampler_fuse_views_loss) in place of the sampler, the fused loss and the sampler's flow
+    gradient; the sources get no gradient: it raises if ``data`` needs one."""
+    views, flags = _views_args(data, head, views, grid_order, target)
+    if torch.is_grad_enabled() and data.requires_grad:
+        raise RuntimeError("fused_views_warp_loss has no gradient wrt the sources: pass sources that need no gradient")
+    Cc = data.shape[-1]
+    weights = [1.0] * Cc if weights is None else list(weights)
+    if inv_count is None:
+        inv_count = 1.0 / (target.numel() // Cc)
+    want_grad = torch.is_grad_enabled() and head.requires_grad
+    return _ViewsWarpLoss.apply(data.contiguous(), head.contiguous(), target.contiguous(), views, flags, tuple(weights), mode, inv_count,
+                                unit_upstream, want_grad)
+
+
+def fused_views_warp(data, head, views, grid_order="ref_yx"):
+    """Forward only of fused_views_warp_loss: data [views*B,H,W,C], head [views*B,Hout,Wout,3] -> fused [B,Hout,Wout,C]."""
+    views, flags = _views_args(data, head, views, grid_order)
+    data, head = data.contiguous(), head.contiguous()
+    B, Cc = data.shape[0] // views, data.shape[-1]
+    Ho, Wo = head.shape[1], head.shape[2]
+    fused = torch.empty((B, Ho, Wo, Cc), dtype=torch.float32, device=data.device)
+    _tag[0] = "sampler"
+    call("dmv_sampler_fuse_views_loss", _p(data), views, _p(head), None, None, 0, 0.0, _p(fused), None, None, B, data.shape[1],
+         data.shape[2], Cc, Ho, Wo, flags, None, 0, _stream(data))
+    return fused
+
+
 def resampler_debug(data, wf, flags=0):
     """Forward plus the bit-exact targets: corner indices [.,4] int32 and predicate mask uint8."""
     _need_cuda(data, wf)

@@ -40,6 +40,9 @@ class Base_Prediction_Model(ModelBase):
         self.num_targets = int(conf.get("num_targets", 1))
         if self.num_targets < 1:
             raise ValueError("num_targets must be >= 1")
+        if int(conf.get("num_views", 1)) > 1:
+            raise ValueError("%s takes one source view per target (num_views = %s): its colour and depth heads have "
+                             "no confidence channel to fuse several views by" % (type(self).__name__, conf["num_views"]))
         self.grid_order = conf.get("grid_order", "ref_yx")
         self.algo = conf.get("algo", None)
         self.use_color = "use_color" in conf

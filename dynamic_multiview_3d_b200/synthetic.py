@@ -8,6 +8,7 @@ the reference-native (d_elevation, d_azimuth) radians (collect_data_node.py:125-
 targets=T > 1: T target views per source at distinct azimuth bins, image1 [B, T, H, W, 3], disp [B, T, V] (depth1 /
 mask1 likewise).  Target 0 and everything else are the targets=1 batch of the same seed; the other targets are drawn
 after it.
+make_multiview_batch: several source views of one car per target (the single-view models' num_views).
 Host-side NumPy: this is input generation, not part of the measured path.
 """
 import numpy as np
@@ -95,6 +96,50 @@ def _more_targets(rng, blob, scenes, bins, T, viewpoint, image1, depth1, mask1, 
     im[:, 1:] += rng.normal(0, 0.02, im[:, 1:].shape).astype(np.float32)
     np.clip(im, 0, 1, out=im)
     return im, dp, mk, ds
+
+
+def make_multiview_batch(batch, size=224, views=2, viewpoint="onehot19", seed=1234, rank=0):
+    """Several source views of one car per target (AppearanceFlowModel with num_views): image0 [views, B, H, W, 3],
+    disp [views, B, V], image1 [B, H, W, 3].  Source v of sample b shows the car rotated by bins[v, b] * 20 degrees less
+    than the target, at an azimuth bin distinct from the sample's other sources; its disp row is that rotation to the
+    target: the one-hot bin, or (0, d_azimuth) radians."""
+    if not 1 <= views <= 19:
+        raise ValueError("views must be 1 .. 19 (one per azimuth bin), got %d" % views)
+    rng = np.random.default_rng(seed + rank)
+    H = W = size
+    yy, xx = np.mgrid[0:H, 0:W].astype(np.float32)
+    cy, cx = (H - 1) / 2.0, (W - 1) / 2.0
+
+    def blob(yaw, colour, jitter):
+        c, s = np.cos(yaw), np.sin(yaw)
+        u = ((xx - cx - jitter[0]) * c + (yy - cy - jitter[1]) * s) / (0.275 * W)
+        v = (-(xx - cx - jitter[0]) * s + (yy - cy - jitter[1]) * c) / (0.125 * H)
+        img = np.full((H, W, 3), 0.5, np.float32)
+        img[(u * u + v * v) <= 1.0] = colour
+        return img
+
+    image0 = np.empty((views, batch, H, W, 3), np.float32)
+    image1 = np.empty((batch, H, W, 3), np.float32)
+    disp = np.zeros((views, batch, 19 if viewpoint == "onehot19" else 2), np.float32)
+    bins = np.empty((views, batch), np.int64)
+    for b in range(batch):
+        colour = rng.uniform(0.1, 0.9, size=3).astype(np.float32)
+        jit = rng.uniform(-4, 4, size=2)
+        yaw1 = rng.uniform(0, 2 * np.pi)
+        image1[b] = blob(yaw1, colour, jit)
+        bins[:, b] = rng.choice(19, size=views, replace=False)
+        for v in range(views):
+            daz = np.deg2rad(20.0 * bins[v, b])
+            image0[v, b] = blob(yaw1 - daz, colour, jit)
+            if viewpoint == "onehot19":
+                disp[v, b, bins[v, b]] = 1.0
+            else:
+                disp[v, b] = (0.0, daz)
+    image0 += rng.normal(0, 0.02, image0.shape).astype(np.float32)
+    image1 += rng.normal(0, 0.02, image1.shape).astype(np.float32)
+    np.clip(image0, 0, 1, out=image0)
+    np.clip(image1, 0, 1, out=image1)
+    return {"image0": image0, "image1": image1, "disp": disp, "bins": bins}
 
 
 def make_multiobject_batch(batch, size=128, seed=1234, rank=0):

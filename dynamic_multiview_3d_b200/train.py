@@ -319,6 +319,8 @@ def synthetic_batch(model, seed, rank=0):
         b = S.make_multiview_multiobject_batch(B, H, model.num_views, seed=seed, rank=rank, viewpoint=vp)
     elif isinstance(model, MultiObjectAppFlow):
         b = S.make_multiobject_batch(B, H, seed=seed, rank=rank)
+    elif getattr(model, "num_views", 1) > 1:
+        b = S.make_multiview_batch(B, H, model.num_views, vp, seed=seed, rank=rank)
     else:
         b = S.make_batch(B, H, vp, seed=seed, rank=rank, depth=True, targets=getattr(model, "num_targets", 1))
     return {k: b[k] for k in model.INPUT_KEYS}
@@ -373,6 +375,12 @@ def main(argv=None):
         raise SystemExit("--tfrecords trains one target per source: each record holds one (source, target) pair and names no "
                          "object, so records cannot be grouped into several targets of one source; set num_targets = 1 or "
                          "train on synthetic batches")
+    from .appearance_flow_model import AppearanceFlowModel
+    if args.tfrecords and int(conf.get("num_views", 1)) > 1 and isinstance(conf.get("model"), type) \
+            and issubclass(conf["model"], AppearanceFlowModel):
+        raise SystemExit("--tfrecords trains one source view per target with %s: each record holds one (source, target) pair, "
+                         "so records cannot be grouped into several views of one target; set num_views = 1 or train on "
+                         "synthetic batches" % conf["model"].__name__)
     if world > 1:
         import torch.distributed as dist
         torch.cuda.set_device(local)

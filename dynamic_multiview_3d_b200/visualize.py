@@ -224,11 +224,12 @@ def visualize_multiview(model, batch, iter_num=None):
     return {"loss": loss, "max_resample_coord": float("nan"), "mean_confidence": [float(w.mean()) for w in wts]}
 
 
-def visualize(model, image0, image1, disp, iter_num=None, seed=0):
+def visualize(model, image0, image1, disp, iter_num=None, seed=0, source=None):
     """appearance_flow_model.py:132-179 for a model with (image0, disp) -> gen.  Writes output_/tr_gt_/tr_input_<iter>.png
     (8x8 grids), quiver_<iter>.png and corr_plot_<iter>.png (the reference's two figures, rasterised), flow_<iter>.png
     (sample 0 as a colour-wheel image) and returns {'loss', 'max_resample_coord', 'correspondences':
-    [(output_pt, sampled_location)] * 6}."""
+    [(output_pt, sampled_location)] * 6}.  ``source`` [B,H,W,3]: the input the grids and the correspondence plot show when
+    it is not image0 itself (source frame 0 of a model with several source views)."""
     import torch
     if iter_num is None:
         m = re.match(".*?([0-9]+)$", str(model.conf.get("visualize", "0")))
@@ -242,13 +243,15 @@ def visualize(model, image0, image1, disp, iter_num=None, seed=0):
     warp_pts = model.warp_pts.cpu().numpy()
     save_images(gen, [8, 8], os.path.join(path, "output_%s.png" % iter_num))
     save_images(image1.detach().cpu().numpy(), [8, 8], os.path.join(path, "tr_gt_%s.png" % iter_num))
-    save_images(image0.detach().cpu().numpy(), [8, 8], os.path.join(path, "tr_input_%s.png" % iter_num))
-    write_png(os.path.join(path, "flow_%s.png" % iter_num), flow_to_color(model.flow_field[0].detach().float().cpu().numpy()))
+    shown = image0 if source is None else source
+    save_images(shown.detach().cpu().numpy(), [8, 8], os.path.join(path, "tr_input_%s.png" % iter_num))
+    flow = model.flow_field.reshape((-1,) + tuple(model.flow_field.shape[-3:]))
+    write_png(os.path.join(path, "flow_%s.png" % iter_num), flow_to_color(flow[0].detach().float().cpu().numpy()))
     H = gen.shape[1]
     rng = np.random.RandomState(seed)
     pts = rng.randint(int(0.3125 * H), int(0.6875 * H), size=(6, 2))           # randint(40, 88) at 128 (:166)
     corr = [(tuple(int(v) for v in p), tuple(int(v) for v in warp_pts[0, p[0], p[1], :].astype("uint32"))) for p in pts]
     write_png(os.path.join(path, "quiver_%s.png" % iter_num), quiver_image(warp_pts[0]))
     write_png(os.path.join(path, "corr_plot_%s.png" % iter_num),
-              corr_plot_image(image0[0].detach().cpu().numpy(), gen[0], [c[0] for c in corr], [c[1] for c in corr]))
+              corr_plot_image(shown[0].detach().cpu().numpy(), gen[0], [c[0] for c in corr], [c[1] for c in corr]))
     return {"loss": loss, "max_resample_coord": float(np.max(warp_pts)), "correspondences": corr}

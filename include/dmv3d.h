@@ -148,6 +148,27 @@ int dmv_sampler_loss_fused(const float* data, const float* wf, const float* targ
                            int W, int C, int Hout, int Wout, unsigned flags, void* workspace,
                            size_t workspace_bytes, void* stream);
 
+/* Several source views per target (Zhou et al.'s multi-view appearance flow) in ONE kernel: each view's warp, the
+ * confidence-weighted fusion, the loss and the gradient wrt the 3-channel head.  View v of target b is row v*B + b:
+ *   data   [views*B,H,W,C] f32      head [views*B,Hout,Wout,3] f32: channels 0-1 the flow (grid added per flags, as
+ *                                   dmv_sampler_fwd), channel 2 the confidence logit; read in place
+ *   target [B,Hout,Wout,C] f32, or NULL: forward only (fused_out required, grad_head and loss_out NULL)
+ *   fused_out [B,Hout,Wout,C] = sum_v softmax_v(logit) * warp(src_v, flow_v), or NULL
+ *   grad_head [views*B,Hout,Wout,3] = (dL/dflow, dL/dlogit), written whole (channel 2 is 0 for views == 1), or NULL
+ *             (a validation pass: loss only)
+ *   loss_out  device float[1] as dmv_loss_fused_fwd_bwd (no mask)
+ * fused_out and grad_head have the bits of dmv_sampler_fwd per view, dmv_loss_fused_fwd_bwd (V = views, the logits) and
+ * the grad_wf half of dmv_sampler_bwd on its grad_gen.  The loss is a deterministic per-CTA sum (same inputs -> same
+ * bits; within 1e-6 relative of the composition's, which sums in another order).  1 <= views <= 8, C in {1,3,4}, W*C and
+ * Wout*C multiples of 4, Hout > 1, 16-byte aligned buffers.  workspace (training only):
+ * dmv_sampler_loss_workspace_size(B, Hout, Wout) bytes, zeroed once, not shared between concurrent calls.
+ * Refusals launch nothing: DMV_E_INVALID_ARG for a null data / head, a NULL combination the mode does not allow, or an
+ * unknown loss mode; DMV_E_UNSUPPORTED_SHAPE for views, C or the shape; DMV_E_ALIGN; DMV_E_WORKSPACE.                */
+int dmv_sampler_fuse_views_loss(const float* data, int views, const float* head, const float* target,
+                                const float* chan_weight, int mode, float inv_count, float* fused_out, float* grad_head,
+                                float* loss_out, int B, int H, int W, int C, int Hout, int Wout, unsigned flags,
+                                void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- fused loss (+ multi-view confidence fusion) forward and backward ----------------- *
  * replaces euclidean_loss / l1_loss (tf_utils.py:18-23) and the weighted sums of
  * main_model.py:144-154, multiobject_appflow.py:223-283, plus their gradients.
