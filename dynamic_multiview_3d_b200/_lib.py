@@ -32,6 +32,7 @@ SIGNATURES = {
     "dmv_sampler_bwd_workspace_size": (_sz, [_i, _i, _i, _i, _i, _i]),
     "dmv_sampler_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _u, _vp, _sz, _vp]),
     "dmv_sampler_loss_workspace_size": (_sz, [_i, _i, _i]),
+    "dmv_ssim_loss_fwd_bwd": (_i, [_vp, _vp, _vp, _f, _f, _vp, _vp, _i, _i, _i, _i, _vp, _sz, _vp]),
     "dmv_sampler_loss_fused": (_i, [_vp, _vp, _vp, C.POINTER(_f), _i, _f, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _u, _vp, _sz, _vp]),
     "dmv_sampler_loss_fused_shared_src": (_i, [_vp, _i, _i, _vp, _vp, C.POINTER(_f), _i, _f, _vp, _vp, _vp, _i, _i, _i, _i, _i, _u, _vp, _sz, _vp]),
     "dmv_sampler_grad_flow_shared_src": (_i, [_vp, _i, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _u, _vp]),

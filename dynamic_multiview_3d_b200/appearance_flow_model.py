@@ -14,7 +14,8 @@ of SURVEY.md 8(a) (side H multiple of 32, bottleneck H/32), so conf['image_size'
 reproduces the reference shapes and 224 gives BASELINE's.
 
 Extra conf keys (all optional): image_size (128), viewpoint_dim (2), loss ('l2' = reference,
-'l1' = north-star), grid_order ('ref_yx' = the reference's transposing (Y,X) grid, 'xy'),
+'l1' = north-star, 'ssim' = alpha (1 - SSIM) / 2 + (1 - alpha) |d| with alpha = ssim_alpha (0.85); not with num_views > 1),
+grid_order ('ref_yx' = the reference's transposing (Y,X) grid, 'xy'),
 algo ('auto'|'simt'|'tcgen05'), seed (0), num_targets (1), num_views (1).
 
 Several targets per source: a batch with disp [B, T, viewpoint_dim] and image1 [B, T, H, H, 3] trains B sources x T
@@ -67,6 +68,10 @@ class AppearanceFlowModel(ModelBase):
         self.head_channels = 3 if self.num_views > 1 else 2      # flow, plus the confidence logit with several views
         self.confidence = None
         self.loss_mode = conf.get("loss", "l2")
+        self.ssim_alpha = float(conf.get("ssim_alpha", 0.85))
+        if self.loss_mode == "ssim" and self.num_views > 1:
+            raise ValueError("%s with num_views = %d has no 'ssim' loss: the multi-view kernel fuses the views before the loss "
+                             "and has no SSIM form; use 'l2' or 'l1'" % (type(self).__name__, self.num_views))
         self.grid_order = conf.get("grid_order", "ref_yx")
         self.algo = conf.get("algo", None)
         self.max_iter = 1000000
@@ -238,12 +243,13 @@ class AppearanceFlowModel(ModelBase):
         The mean runs over the GLOBAL batch under data parallelism."""
         self.image1 = image1
         n = image1.numel() // image1.shape[-1] * self.world_size       # every target pixel: B*H*W (B*T*H*W with T targets)
-        self.loss = F.reconstruction_loss(self.gen, image1, self.loss_mode, inv_count=1.0 / n, unit_upstream=True)
+        self.loss = F.reconstruction_loss(self.gen, image1, self.loss_mode, inv_count=1.0 / n, unit_upstream=True, **self._ssim_kw())
         return self.loss
 
     def forward_and_loss(self, image0, image1, disp):
         """forward + build_loss with the warp, the loss and the flow gradient fused into one kernel (the training
-        path).  Falls back to the separate calls for shapes the fused kernel does not cover."""
+        path).  Falls back to the separate calls for shapes the fused kernel does not cover and for loss 'ssim', which has no
+        fused form."""
         if type(self).forward is not AppearanceFlowModel.forward or type(self).build_loss is not AppearanceFlowModel.build_loss \
                 or self.device.type == "meta":
             self.forward(image0, disp)
@@ -257,7 +263,7 @@ class AppearanceFlowModel(ModelBase):
         self.image0, self.disp, self.image1 = image0, disp, image1
         with use_store(self.store):
             self.flow_field = self.buildModel(image0, F.to_bf16(disp))
-        if not F.warp_loss_supported(image0, self.flow_field, image1) or os.environ.get("DMV_NO_WARP_LOSS"):
+        if not F.warp_loss_supported(image0, self.flow_field, image1, self.loss_mode) or os.environ.get("DMV_NO_WARP_LOSS"):
             with use_store(self.store):
                 self.gen = flow_resample_layer(image0, self.flow_field, self.grid_order)
             return self.build_loss(image1)
@@ -275,7 +281,7 @@ class AppearanceFlowModel(ModelBase):
         with use_store(self.store):
             flow, T = self._grouped_flow(image0, disp)
         target = image1.reshape((flow.shape[0],) + tuple(image1.shape[2:]))
-        if not F.warp_loss_supported(image0, flow, target) or os.environ.get("DMV_NO_WARP_LOSS"):
+        if not F.warp_loss_supported(image0, flow, target, self.loss_mode) or os.environ.get("DMV_NO_WARP_LOSS"):
             self.flow_field = _per_source(flow, T)
             self.gen = _per_source(F.flow_resampler_grouped(image0, flow, T, self.grid_order), T)
             return self.build_loss(image1)

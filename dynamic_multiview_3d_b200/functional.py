@@ -985,14 +985,17 @@ def _passed_aligned16(t):
     return not t.is_contiguous() or t.data_ptr() % 16 == 0
 
 
-def warp_loss_supported(data, flow, target=None):
-    """True exactly when dmv_sampler_loss_fused accepts the call ``flow_resample_loss(data, flow, target)`` makes: C in
-    {1,3,4}, W*C and Wout*C multiples of 4, an image-shaped flow (Hout > 1) and 16-byte aligned source, flow and target.
+def warp_loss_supported(data, flow, target=None, mode="l2"):
+    """True exactly when dmv_sampler_loss_fused accepts the call ``flow_resample_loss(data, flow, target, mode)`` makes:
+    C in {1,3,4}, W*C and Wout*C multiples of 4, an image-shaped flow (Hout > 1) and 16-byte aligned source, flow and
+    target.  Never for mode 'ssim': the SSIM + L1 loss has no fused warp form (a fused kernel measured no faster than the
+    sampler, ssim_l1_loss and the sampler's flow gradient as separate calls), so its callers take those calls.
     The C ABI returns DMV_E_UNSUPPORTED_SHAPE otherwise, so a caller with a view at an offset must take the separate calls.
     Without ``target`` only the source and the flow are checked: pass the target wherever it is known."""
     Cc, W, Wo = data.shape[-1], data.shape[2], flow.shape[2]
     return (flow.dim() == 4 and data.numel() > 0 and flow.numel() > 0 and flow.shape[1] > 1 and Cc in (1, 3, 4)
             and (W * Cc) % 4 == 0 and (Wo * Cc) % 4 == 0
+            and mode in LOSS
             and all(_passed_aligned16(t) for t in (data, flow, target) if t is not None))
 
 
@@ -1170,10 +1173,55 @@ def _loss_ws(device, nbytes):
     return ws
 
 
-def reconstruction_loss(gen, target, mode="l2", weights=None, inv_count=None, mask=None, unit_upstream=False):
-    """mean_{b,h,w} sum_c w_c * (d^2 | |d|), d = (gen - target) * mask; gradient fused in.
+class _SsimLoss(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, gen, target, weights, alpha, inv_count, unit_upstream):
+        _need_cuda(gen, target)
+        gen, target = gen.contiguous(), target.contiguous()
+        H, W, Cc = gen.shape[-3], gen.shape[-2], gen.shape[-1]
+        B = gen.numel() // (H * W * Cc)
+        w = (C.c_float * Cc)(*[float(x) for x in weights])
+        loss = torch.empty((), dtype=torch.float32, device=gen.device)
+        gg = torch.empty_like(gen) if ctx.needs_input_grad[0] else None
+        ws = _loss_ws(gen.device, _lib.load().dmv_loss_workspace_size(B * H * W))
+        _tag[0] = "loss"
+        call("dmv_ssim_loss_fwd_bwd", _p(gen), _p(target), w, float(alpha), float(inv_count), _p(loss), _p(gg), B, H, W, Cc, _p(ws),
+             ws.numel(), _stream(gen))
+        ctx.gg, ctx.unit_upstream = gg, unit_upstream
+        return loss
+
+    @staticmethod
+    def backward(ctx, gloss):
+        gg = ctx.gg
+        if not ctx.unit_upstream:
+            _tag[0] = "loss"
+            call("dmv_scale_by_device_scalar", _p(gg), _p(gloss.contiguous().to(torch.float32)), gg.numel(), _stream(gg))
+        return gg, None, None, None, None, None
+
+
+def ssim_l1_loss(gen, target, alpha=0.85, weights=None, inv_count=None, unit_upstream=False, mask=None):
+    """inv_count * sum_{images, pixels, c} w_c * (alpha * (1 - SSIM) / 2 + (1 - alpha) * |gen - target|) with a 3x3 SSIM
+    window over reflection-padded images (Monodepth2's SSIM without its clamp; include/dmv3d.h states it in full).
+    gen and target are [..., H, W, C] with H, W >= 2 and C in {1,3,4}; leading axes are images.  inv_count defaults to
+    1 / (images * H * W).  One launch (dmv_ssim_loss_fwd_bwd) with the gradient wrt gen fused in; no mask."""
+    if mask is not None:
+        raise ValueError("ssim_l1_loss takes no mask: a 3x3 window over masked pixels has no defined SSIM here")
+    if gen.shape != target.shape or gen.dim() < 3:
+        raise ValueError("gen and target must both be [..., H, W, C], got %s and %s" % (tuple(gen.shape), tuple(target.shape)))
+    Cc = gen.shape[-1]
+    weights = [1.0] * Cc if weights is None else list(weights)
+    if inv_count is None:
+        inv_count = 1.0 / (target.numel() // Cc)
+    return _SsimLoss.apply(gen, target, tuple(weights), float(alpha), inv_count, unit_upstream)
+
+
+def reconstruction_loss(gen, target, mode="l2", weights=None, inv_count=None, mask=None, unit_upstream=False, alpha=0.85):
+    """mean_{b,h,w} sum_c w_c * (d^2 | |d|), d = (gen - target) * mask; gradient fused in.  mode 'ssim': ssim_l1_loss
+    with ``alpha`` (no mask).
     unit_upstream=True: the loss enters the optimised objective with coefficient 1 (fold other coefficients
     into ``weights``), so backward skips the pass that chains the upstream scalar."""
+    if mode == "ssim":
+        return ssim_l1_loss(gen, target, alpha, weights, inv_count, unit_upstream, mask)
     Cc = gen.shape[-1]
     weights = [1.0] * Cc if weights is None else list(weights)
     if inv_count is None:

@@ -9,7 +9,8 @@ loss = L(colour) + depth_lr_factor * L(depth) (:144-154).
 
 Feature switches are key-presence tests on ``conf`` as in the reference (``'use_color' in conf``).
 Extensions (optional conf keys): image_size (128), viewpoint_dim (2), loss ('l2' reference | 'l1' per-channel L1,
-tf_utils.py:22), head ('tanh' reference | 'flow': each head emits a 2-channel flow and the output is the bilinear
+tf_utils.py:22 | 'ssim' SSIM + L1 with weight ssim_alpha (0.85) on SSIM, functional.ssim_l1_loss), head ('tanh' reference |
+'flow': each head emits a 2-channel flow and the output is the bilinear
 warp of its source modality -- the north-star's "warped RGB/depth"; precedent: multiobject_appflow.py:191-209),
 grid_order, algo, seed, num_targets (1).  The reference ignores conf['batch_size'] (main_model.py:19 hard-codes 64); here
 conf wins.  Several targets per source (disp [B, T, V], image1 / depth1 [B, T, H, H, C]) train as the appearance-flow
@@ -36,6 +37,7 @@ class Base_Prediction_Model(ModelBase):
         self.image_shape = [H, H, 3]
         self.viewpoint_dim = int(conf.get("viewpoint_dim", 2))
         self.loss_mode = conf.get("loss", "l2")
+        self.ssim_alpha = float(conf.get("ssim_alpha", 0.85))
         self.head = conf.get("head", "tanh")
         self.num_targets = int(conf.get("num_targets", 1))
         if self.num_targets < 1:
@@ -185,10 +187,12 @@ class Base_Prediction_Model(ModelBase):
         n = image1.numel() // image1.shape[-1] * self.world_size       # every target pixel: B*H*W (B*T*H*W with T targets)
         loss = None
         if self.use_color:
-            loss = F.reconstruction_loss(self.gen_image1, image1, self.loss_mode, inv_count=1.0 / n, unit_upstream=True)
+            loss = F.reconstruction_loss(self.gen_image1, image1, self.loss_mode, inv_count=1.0 / n, unit_upstream=True,
+                                         **self._ssim_kw())
         if self.use_depth:
             f = float(self.conf["depth_lr_factor"])
-            ld = F.reconstruction_loss(self.gen_dimage1, dimage1, self.loss_mode, weights=[f], inv_count=1.0 / n, unit_upstream=True)
+            ld = F.reconstruction_loss(self.gen_dimage1, dimage1, self.loss_mode, weights=[f], inv_count=1.0 / n, unit_upstream=True,
+                                       **self._ssim_kw())
             loss = ld if loss is None else loss + ld
         self.image1, self.dimage1, self.loss = image1, dimage1, loss
         return loss

@@ -37,6 +37,10 @@ class ModelBase(object):
         """forward + loss on the training path; returns the scalar loss tensor (with its tape)."""
         raise NotImplementedError
 
+    def _ssim_kw(self):
+        """Extra keyword of the loss calls under conf['loss'] = 'ssim' (the weight of the SSIM term); 'l2' / 'l1' take none."""
+        return {"alpha": self.ssim_alpha} if self.loss_mode == "ssim" else {}
+
     def train_step(self, *args):
         """One sess.run([loss, train_op]) of train.py:122: forward, backward, (gradient exchange,) Adam."""
         dp = getattr(self, "_dp", None)

@@ -252,6 +252,9 @@ class MultiViewFusionAppFlow(MultiObjectAppFlow):
     def __init__(self, conf, load_tfrec=True, build_loss=True, device=None):
         self.num_views = int(conf.get("num_views", 4))
         self.loss_mode = conf.get("loss", "l2")
+        if self.loss_mode == "ssim":
+            raise ValueError("%s has no 'ssim' loss: its kernel fuses the views before the loss and has no SSIM form; use 'l2' "
+                             "or 'l1'" % type(self).__name__)
         self.gens = self.logits = self.fused = self.flow_field = None
         conf = dict(conf)
         conf.setdefault("use_color", "")

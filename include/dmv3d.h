@@ -189,6 +189,24 @@ int dmv_loss_fused_fwd_bwd(const float* gen, const float* logits, int V, const f
                            float* grad_logits, float* fused_out, long long pixels, int C,
                            void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- SSIM + L1 photometric loss (Monodepth / SfMLearner-style) ----------------------------------------------- *
+ * Per image and channel, with x = gen and y = target reflection-padded by one pixel (row -1 reads row 1, row H reads
+ * row H-2, the same for columns) and the 3x3 window centred on every pixel p:
+ *   SSIM_p = ((2 mu_x mu_y + C1)(2 s_xy + C2)) / ((mu_x^2 + mu_y^2 + C1)(s_xx + s_yy + C2)),  C1 = 0.01^2, C2 = 0.03^2,
+ *   s_xx = mean(x^2) - mu_x^2, s_xy = mean(xy) - mu_x mu_y   (Monodepth2's SSIM without its final clamp)
+ *   loss_out = inv_count * sum_{n,p} sum_c w_c * (alpha * (1 - SSIM_p,c) / 2 + (1 - alpha) * |x - y|)
+ * alpha = 0 is the L1 loss; d|d|/dd = 0 at d = 0.  The loss is a deterministic per-CTA sum (same inputs -> same bits).
+ *   gen, target, grad_gen [B,H,W,C] f32; grad_gen = d loss / d gen, or NULL (loss only: a validation pass)
+ *   chan_weight host float[C]; workspace dmv_loss_workspace_size(B*H*W) bytes, 8-byte aligned, zeroed once and not
+ *   shared between concurrent calls.  Launches one kernel (label "loss_fused").
+ * Refusals launch nothing: DMV_E_INVALID_ARG for a null pointer or alpha outside [0, 1] or NaN; DMV_E_UNSUPPORTED_SHAPE
+ * for C not in {1,3,4}, B < 1 or H, W < 2; DMV_E_WORKSPACE; DMV_E_ALIGN for an unaligned workspace.
+ * There is no fused warp + SSIM form: warp with dmv_sampler_fwd, take this loss, and the flow gradient with the grad_wf
+ * half of dmv_sampler_bwd (a fused kernel measured no faster than these three calls; DESIGN.md §4).               */
+int dmv_ssim_loss_fwd_bwd(const float* gen, const float* target, const float* chan_weight, float alpha, float inv_count,
+                          float* loss_out, float* grad_gen, int B, int H, int W, int C, void* workspace,
+                          size_t workspace_bytes, void* stream);
+
 /* x[i] *= *scalar (device scalar): chains an upstream loss gradient without a host sync */
 int dmv_scale_by_device_scalar(float* x, const float* scalar, long long n, void* stream);
 
